@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - RQ-KMeans vectors/sec per iteration (512-d, [128,128,256]) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--rows R] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[1]): 1M x 512 fp32 synthetic vectors per GPU (weak scaling: the fit is
@@ -326,12 +326,14 @@ class Workload:
                 cur = engine.residual_normalise(cur, ids, km.cluster_centers, [DIM])
         self.bufs = [None] * len(self.levels)
         self.stats = []
+        self.last = None
 
     def step(self, i):
         import torch
         lvl = i % len(self.levels)
         km, xl = self.levels[lvl]
-        score, _assign, stats, _shift = km._iterate(xl, self.n_global, self.bufs[lvl])
+        score, assign, stats, shift = km._iterate(xl, self.n_global, self.bufs[lvl])
+        self.last = (lvl, score, assign, shift)
         self.bufs[lvl] = score.scores_t
         c = score.counts.to(torch.int64)
         if self.shard is not None:
@@ -372,6 +374,32 @@ class Workload:
                 "list_rounds_per_step": [st.list_passes for _, st in self.stats],
                 "window_misses_per_step": [st.window_misses for _, st in self.stats],
                 "reference_rounds_per_step": [st.rounds for _, st in self.stats], "peak_source": how}
+
+    def dump(self, out_dir, max_rows=1 << 20, score_rows=4096):
+        """Writes what the last timed step returned to its caller as DIR/<name>.npy, so that two builds can be
+        compared output for output: the updated centres, the balanced assignment, the argmin and counts of the
+        step's input centres, the centre shift, and the fp16 scores of `score_rows` rows.  Per-row outputs of more
+        than `max_rows` rows are a fixed sample (rows.npy holds its row indices); everything stays under 64 MB."""
+        import numpy as np
+        import torch
+        lvl, score, assign, shift = self.last
+        km = self.levels[lvl][0]
+        n = self.n
+        rows = np.arange(n) if n <= max_rows else np.sort(np.random.default_rng(0).choice(n, max_rows, replace=False))
+        out = {"centers": km.cluster_centers.cpu().numpy().astype(np.float32),
+               "assignment": assign.cpu().numpy()[rows].astype(np.float64),
+               "argmin": score.argmin.cpu().numpy()[rows].astype(np.float64),
+               "counts": score.counts.cpu().numpy().astype(np.float64),
+               "shift": np.array([shift], dtype=np.float64)}
+        if n > max_rows:
+            out["rows"] = rows.astype(np.float64)
+        if score.scores_t is not None:
+            cols = np.sort(np.random.default_rng(1).choice(n, min(n, score_rows), replace=False))
+            s = score.scores_t.index_select(1, torch.from_numpy(cols).to(score.scores_t.device))
+            out["scores"] = s.t().float().cpu().numpy()
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in out.items():
+            np.save(os.path.join(out_dir, f"{name}.npy"), a)
 
 
 def fit_10m_record(dev, engine, KMeans, peak, how, rows=10000000, iters=3):
@@ -453,8 +481,14 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-10m", action="store_true", help="skip the 10 M-row single-GPU record")
     ap.add_argument("--no-extras", action="store_true", help="only the headline step timing (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0's rows) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs dumps the GPU step; it does not apply to --impl reference")
         return run_reference(args)
     if args.no_extras:
         args.no_e2e = args.no_cpu = args.no_10m = True
@@ -489,6 +523,8 @@ def main():
         sampler.start()                                      # before the warm-up: it is streaming when the timed region starts
     ms = wl.timed(args.warmup, args.steps, barrier, sampler if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        wl.dump(args.dump_outputs)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
