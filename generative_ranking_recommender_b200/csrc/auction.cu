@@ -63,6 +63,8 @@ constexpr int AUC_SUB = 4096;      // jobs whose cost / owner are staged in shar
 constexpr int AUC_QCAP = 256;      // per-warp survivor queue of the HIST kernel (one row segment; = AUC_SEG_CAP)
 constexpr int AUC_SAMPLE_MAX = 8192; // window-sampling jobs per worker (all ranks together)
 constexpr int AUC_SEG_CAP = 256;   // survivor-list entries per (sub-range, worker); ~60 expected
+constexpr int AUC_KH = 128;        // workers per histogram half of the HIST kernel
+constexpr int AUC_SAMPLE_THREADS = 512; // threads of a window-sampling CTA (2 CTAs per SM: K = 256 in one wave)
 
 enum { MODE_HIST = 0, MODE_BID = 1, MODE_DONE = 2 };
 
@@ -718,8 +720,9 @@ __device__ __forceinline__ void hist_add(unsigned int* hist, int w, int bin, uns
 
 // Window geometry.  shift > 0: 128 contiguous bins of 2^shift keys from `base`.  shift == 0: one-key bins,
 // bins 0..nlo-1 = [base, base+nlo), bins nlo..127 = [hbase, hbase+128-nlo), hbase >= base+nlo; keys in
-// between are counted in `gap`, keys above in `above`, keys below `base` are ignored.
-__device__ __forceinline__ void window_count(const PassSmem& sm, int w, int key) {
+// between are counted in `gap`, keys above in `above`, keys below `base` are ignored.  Worker w's histogram is row
+// `hrow` of sm.hist.
+__device__ __forceinline__ void window_count(const PassSmem& sm, int w, int hrow, int key) {
     const int base = sm.r_base[w];
     const int shift = sm.r_shift[w];
     if (key < base) return;
@@ -727,16 +730,16 @@ __device__ __forceinline__ void window_count(const PassSmem& sm, int w, int key)
         const int hb = sm.r_hbase[w], nlo = sm.r_nlo[w];
         if (key >= hb) {
             if (key - hb >= AUC_W - nlo) atomicAdd(&sm.above[w], 1u);
-            else hist_add(sm.hist, w, nlo + key - hb);
+            else hist_add(sm.hist, hrow, nlo + key - hb);
         } else if (key >= base + nlo) {
             atomicAdd(&sm.gap[w], 1u);
         } else {
-            hist_add(sm.hist, w, key - base);
+            hist_add(sm.hist, hrow, key - base);
         }
     } else {
         const int bin = (key - base) >> shift;
         if (bin >= AUC_W) atomicAdd(&sm.above[w], 1u);
-        else hist_add(sm.hist, w, bin);
+        else hist_add(sm.hist, hrow, bin);
     }
 }
 
@@ -1065,36 +1068,42 @@ __device__ __forceinline__ uint4 ldg_stream128(const void* ptr) {
     return r;
 }
 
-// Shared-memory layout with compile-time offsets (KP = K rounded up to 128 or 256): with run-time offsets the
-// compiler re-derives the array bases inside the hot loops (64 registers per thread leave no room to keep them).
-template <int KP>
+// Shared-memory layout with compile-time offsets: with run-time offsets the compiler re-derives the array bases inside
+// the hot loops (64 registers per thread leave no room to keep them).  The histogram holds one half of the workers
+// (AUC_KH rows, 64 KB, so that two CTAs fit on an SM); the per-worker arrays hold all K <= 256.
 struct HistSmem {
-    static constexpr int HIST = 0;                                    // [KP][W/2] two 16-bit counters per word
-    static constexpr int COST = HIST + KP * AUC_W * 2;                // [HS_SUB] fp16
+    static constexpr int KMAX = 256;
+    static constexpr int HIST = 0;                                    // [AUC_KH][W/2] two 16-bit counters per word
+    static constexpr int COST = HIST + AUC_KH * AUC_W * 2;            // [HS_SUB] fp16
     static constexpr int OWN = COST + HS_SUB * 2;                     // [HS_SUB] int16
     static constexpr int HQ = OWN + HS_SUB * 2;                       // [NW][QCAP] survivor queue
-    static constexpr int ABOVE = HQ + AUC_NW * AUC_QCAP * 2;          // [KP] u32 ...
-    static constexpr int GAP = ABOVE + KP * 4;
-    static constexpr int RBASE = GAP + KP * 4;
-    static constexpr int RHBASE = RBASE + KP * 4;
-    static constexpr int RNLO = RHBASE + KP * 4;
-    static constexpr int RLO2 = RNLO + KP * 4;
-    static constexpr int SEGCNT = RLO2 + KP * 4;
-    static constexpr int ACT = SEGCNT + KP * 4;                       // [KP] u16 unresolved workers, ascending
-    static constexpr int RSHIFT = ACT + KP * 2;                       // [KP] u8 (0xff: resolved by an earlier pass)
-    static constexpr int TOTAL = (RSHIFT + KP + 15) / 16 * 16;
+    static constexpr int ABOVE = HQ + AUC_NW * AUC_QCAP * 2;          // [KMAX] u32 ...
+    static constexpr int GAP = ABOVE + KMAX * 4;
+    static constexpr int RBASE = GAP + KMAX * 4;
+    static constexpr int RHBASE = RBASE + KMAX * 4;
+    static constexpr int RNLO = RHBASE + KMAX * 4;
+    static constexpr int RLO2 = RNLO + KMAX * 4;
+    static constexpr int SEGCNT = RLO2 + KMAX * 4;
+    static constexpr int ACT = SEGCNT + KMAX * 4;                     // [KMAX] u16 unresolved workers, ascending
+    static constexpr int RSHIFT = ACT + KMAX * 2;                     // [KMAX] u8 (0xff: resolved by an earlier pass)
+    static constexpr int TOTAL = (RSHIFT + KMAX + 15) / 16 * 16;
 };
 
-template <int KP>
-__global__ void __launch_bounds__(AUC_THREADS, (KP <= 128 ? 2 : 1))
+// K > AUC_KH: the CTA runs its job range once per half of the workers, [0, 128) then [128, K), with the histogram
+// cleared in between.  That keeps the K = 128 register and shared-memory budget (2 CTAs per SM) for every K; the
+// cost / owner staging is repeated per half (6 bytes per job against 256 bytes of S per job and half).
+__global__ void __launch_bounds__(AUC_THREADS, 2)
 auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int K, int J, int spc, AuctionPtrs p,
                     long long n_global, int fused) {
-    using L = HistSmem<KP>;
+    using L = HistSmem;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     pdl_launch_dependents();
     // nothing below depends on earlier kernels until pdl_wait(): the histogram is cleared while they finish
-    for (int i = threadIdx.x; i < KP * AUC_W * 2 / 16; i += AUC_THREADS)
-        reinterpret_cast<uint4*>(smem_raw)[i] = make_uint4(0u, 0u, 0u, 0u);
+    auto clear_hist = [&] {
+        for (int i = threadIdx.x; i < AUC_KH * AUC_W * 2 / 16; i += AUC_THREADS)
+            reinterpret_cast<uint4*>(smem_raw + L::HIST)[i] = make_uint4(0u, 0u, 0u, 0u);
+    };
+    clear_hist();
     pdl_wait();
     const AuctionState st = *p.st;
     if (st.mode != MODE_HIST) return;
@@ -1114,7 +1123,7 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
     short* const own_s = reinterpret_cast<short*>(smem_raw + L::OWN);
     unsigned int* const seg_cnt_s = reinterpret_cast<unsigned int*>(smem_raw + L::SEGCNT);
     unsigned short* const act = reinterpret_cast<unsigned short*>(smem_raw + L::ACT);
-    __shared__ int s_nact, s_any_cold, s_wcnt[AUC_NW];
+    __shared__ int s_act_off[3], s_any_cold[2], s_wcnt[AUC_NW];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const unsigned int lt = (1u << lane) - 1u;
     unsigned short* const wq = reinterpret_cast<unsigned short*>(smem_raw + L::HQ) + warp * AUC_QCAP;
@@ -1126,8 +1135,9 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
 
     // Rows (workers) of this pass.  A worker whose threshold an earlier pass of the SAME round resolved keeps what
     // that pass produced (threshold, survivor lists, per-CTA dump) and is skipped: after a window miss only the
-    // workers that missed are streamed again, spread over the warps (act[] = the unresolved workers, ascending).
-    if (tid == 0) { s_nact = 0; s_any_cold = 0; }
+    // workers that missed are streamed again, spread over the warps (act[] = the unresolved workers, ascending; those
+    // of half h are act[s_act_off[h] .. s_act_off[h + 1])).
+    if (tid < 2) s_any_cold[tid] = 0;
     for (int i = tid; i < K; i += AUC_THREADS) {
         sm.above[i] = 0;
         sm.gap[i] = 0;
@@ -1149,305 +1159,323 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
         for (int q = 0; q < warp; ++q) off += s_wcnt[q];
         if (a) {
             act[off + __popc(m & lt)] = (unsigned short)tid;
-            if (sm.r_base[tid] <= 0) s_any_cold = 1;
+            if (sm.r_base[tid] <= 0) s_any_cold[tid / AUC_KH] = 1;
         }
-        if (tid == 0) { int t = 0; for (int q = 0; q < AUC_NW; ++q) t += s_wcnt[q]; s_nact = t; }
+        if (tid == 0) {
+            int t = 0;
+            for (int q = 0; q < AUC_NW; ++q) {
+                if (q == AUC_KH / 32) s_act_off[1] = t;
+                t += s_wcnt[q];
+            }
+            s_act_off[0] = 0;
+            s_act_off[2] = t;
+        }
         __syncthreads();
     }
-    const int nact = s_nact;
-    const int any_cold = s_any_cold;                         // cold rows take the unpipelined path
 
-    int seg = b * spc;
-    for (long long sub = c_begin; sub < c_end; sub += HS_SUB, ++seg) {
-        const int sublen = (int)((c_end - sub) < HS_SUB ? (c_end - sub) : HS_SUB);
-        unsigned int* seg_lists = p.seg_list + (size_t)seg * K * AUC_SEG_CAP;
-        if (tid < K) seg_cnt_s[tid] = 0;
-        // ---- stage costs / owners of the sub-range (retain fast-forward applied here, once) ----
-        unsigned short so_r[HS_SUB / AUC_THREADS];   // the owner's own value of my jobs (kept by the BID kernels)
-#pragma unroll
-        for (int it = 0; it < HS_SUB / AUC_THREADS; ++it) {
-            const int i = tid + it * AUC_THREADS;
-            unsigned short c = 0;
-            short o = -1;
-            so_r[it] = 0;
-            if (i < sublen) {
-                __half ch = p.cost[sub + i];
-                o = p.owner[sub + i];
-                so_r[it] = __half_as_ushort(p.sown[sub + i]);
-                if (ff > 0 && o >= 0) {
-                    for (int r = 0; r < ff; ++r) ch = __hadd(ch, eps);
-                    p.cost[sub + i] = ch;
-                }
-                c = __half_as_ushort(ch);
-            }
-            cost_s[i] = c;
-            own_s[i] = o;
+    int ffh = ff;                                            // the retain fast-forward goes to the first half streamed
+    for (int h0 = 0; h0 < K; h0 += AUC_KH) {
+        const unsigned short* const acth = act + s_act_off[h0 / AUC_KH];
+        const int nact = s_act_off[h0 / AUC_KH + 1] - s_act_off[h0 / AUC_KH];
+        if (nact == 0) continue;                                 // every worker of the half was resolved by an earlier pass
+        const int any_cold = s_any_cold[h0 / AUC_KH];            // cold rows take the unpipelined path
+        if (h0 > 0) {
+            __syncthreads();                                     // the previous half's histogram has been published
+            clear_hist();
+            __syncthreads();
         }
-        __syncthreads();
-        // ---- owner entries (value = S): one per job ----
+
+        int seg = b * spc;
+        for (long long sub = c_begin; sub < c_end; sub += HS_SUB, ++seg) {
+            const int sublen = (int)((c_end - sub) < HS_SUB ? (c_end - sub) : HS_SUB);
+            unsigned int* seg_lists = p.seg_list + (size_t)seg * K * AUC_SEG_CAP;
+            if (tid < K) seg_cnt_s[tid] = 0;
+            // ---- stage costs / owners of the sub-range (retain fast-forward applied here, once) ----
+            unsigned short so_r[HS_SUB / AUC_THREADS];   // the owner's own value of my jobs (kept by the BID kernels)
 #pragma unroll
-        for (int it = 0; it < HS_SUB / AUC_THREADS; ++it) {
-            const int i = tid + it * AUC_THREADS;
-            const int o = (i < sublen) ? own_s[i] : -1;
-            if (o >= 0 && sm.r_base[o] > 0 && sm.r_shift[o] != 0xff) {
-                const int key = (int)h2key((unsigned)so_r[it]);
-                window_count(sm, o, key);
-                if (key >= sm.r_base[o]) {
-                    const unsigned int slot = atomicAdd(&seg_cnt_s[o], 1u);
-                    if (slot < AUC_SEG_CAP) seg_lists[(size_t)o * AUC_SEG_CAP + slot] = ((unsigned)i << 16) | (unsigned)key;
+            for (int it = 0; it < HS_SUB / AUC_THREADS; ++it) {
+                const int i = tid + it * AUC_THREADS;
+                unsigned short c = 0;
+                short o = -1;
+                so_r[it] = 0;
+                if (i < sublen) {
+                    __half ch = p.cost[sub + i];
+                    o = p.owner[sub + i];
+                    so_r[it] = __half_as_ushort(p.sown[sub + i]);
+                    if (ffh > 0 && o >= 0) {
+                        for (int r = 0; r < ffh; ++r) ch = __hadd(ch, eps);
+                        p.cost[sub + i] = ch;
+                    }
+                    c = __half_as_ushort(ch);
+                }
+                cost_s[i] = c;
+                own_s[i] = o;
+            }
+            __syncthreads();
+            // ---- owner entries (value = S): one per job, counted in the owner's half ----
+#pragma unroll
+            for (int it = 0; it < HS_SUB / AUC_THREADS; ++it) {
+                const int i = tid + it * AUC_THREADS;
+                const int o = (i < sublen) ? own_s[i] : -1;
+                if (o >= h0 && o < h0 + AUC_KH && sm.r_base[o] > 0 && sm.r_shift[o] != 0xff) {
+                    const int key = (int)h2key((unsigned)so_r[it]);
+                    window_count(sm, o, o - h0, key);
+                    if (key >= sm.r_base[o]) {
+                        const unsigned int slot = atomicAdd(&seg_cnt_s[o], 1u);
+                        if (slot < AUC_SEG_CAP) seg_lists[(size_t)o * AUC_SEG_CAP + slot] = ((unsigned)i << 16) | (unsigned)key;
+                    }
                 }
             }
-        }
-        // One survivor per lane: exact value -> key -> survivor list + window histogram.  Called with all 32 lanes.
-        auto emit = [&](int w, const __half* srow, bool live, int cc, int wbase, int whb, int wnlo, int wshift) {
-            live = live && own_s[cc] != w;                                   // owner entry: counted above
-            int key = 0;
-            if (live) key = (int)h2key(h2bits(__hsub(srow[cc], __ushort_as_half(cost_s[cc]))));
-            const unsigned int m = __ballot_sync(0xffffffffu, live);
-            if (m) {
-                unsigned int slot0 = 0;
-                if (lane == 0) slot0 = atomicAdd(&seg_cnt_s[w], (unsigned)__popc(m));
-                slot0 = __shfl_sync(0xffffffffu, slot0, 0);
-                const unsigned int slot = slot0 + __popc(m & lt);
-                if (live && slot < AUC_SEG_CAP) seg_lists[(size_t)w * AUC_SEG_CAP + slot] = ((unsigned)cc << 16) | (unsigned)key;
-            }
-            if (live) {
-                int bin;
-                if (wshift == 0) bin = key >= whb ? (key - whb >= AUC_W - wnlo ? AUC_W : wnlo + key - whb)
-                                                  : (key >= wbase + wnlo ? -1 : key - wbase);
-                else { bin = (key - wbase) >> wshift; bin = bin > AUC_W ? AUC_W : bin; }
-                if (bin >= AUC_W) atomicAdd(&sm.above[w], 1u);
-                else if (bin < 0) atomicAdd(&sm.gap[w], 1u);
-                else hist_add(sm.hist, w, bin);
-            }
-        };
-        if (!any_cold) {
-            // Fast path (every active row has a fine window).  Software-pipelined: the next step's four 16-byte loads
-            // are in flight while this step is filtered, across row boundaries too.  Survivors are not
-            // handled by the lane that found them (a divergent loop, ~5 of 32 lanes busy) but pushed as
-            // job offsets into a per-warp queue and handled 32 at a time when the queue fills / the row ends.
-            int qn = 0;
-            const int nfull = sublen >> 10, nsteps = (sublen + 1023) >> 10;
-            auto load_step = [&](int w, int st, uint4 (&sv)[4]) {
-                const uint4* rp = reinterpret_cast<const uint4*>(S + (size_t)w * ld + sub) + (st << 7) + lane;
-                if (st < nfull) {
+            // One survivor per lane: exact value -> key -> survivor list + window histogram.  Called with all 32 lanes.
+            auto emit = [&](int w, const __half* srow, bool live, int cc, int wbase, int whb, int wnlo, int wshift) {
+                live = live && own_s[cc] != w;                                   // owner entry: counted above
+                int key = 0;
+                if (live) key = (int)h2key(h2bits(__hsub(srow[cc], __ushort_as_half(cost_s[cc]))));
+                const unsigned int m = __ballot_sync(0xffffffffu, live);
+                if (m) {
+                    unsigned int slot0 = 0;
+                    if (lane == 0) slot0 = atomicAdd(&seg_cnt_s[w], (unsigned)__popc(m));
+                    slot0 = __shfl_sync(0xffffffffu, slot0, 0);
+                    const unsigned int slot = slot0 + __popc(m & lt);
+                    if (live && slot < AUC_SEG_CAP) seg_lists[(size_t)w * AUC_SEG_CAP + slot] = ((unsigned)cc << 16) | (unsigned)key;
+                }
+                if (live) {
+                    int bin;
+                    if (wshift == 0) bin = key >= whb ? (key - whb >= AUC_W - wnlo ? AUC_W : wnlo + key - whb)
+                                                      : (key >= wbase + wnlo ? -1 : key - wbase);
+                    else { bin = (key - wbase) >> wshift; bin = bin > AUC_W ? AUC_W : bin; }
+                    if (bin >= AUC_W) atomicAdd(&sm.above[w], 1u);
+                    else if (bin < 0) atomicAdd(&sm.gap[w], 1u);
+                    else hist_add(sm.hist, w - h0, bin);
+                }
+            };
+            if (!any_cold) {
+                // Fast path (every active row has a fine window).  Software-pipelined: the next step's four 16-byte loads
+                // are in flight while this step is filtered, across row boundaries too.  Survivors are not
+                // handled by the lane that found them (a divergent loop, ~5 of 32 lanes busy) but pushed as
+                // job offsets into a per-warp queue and handled 32 at a time when the queue fills / the row ends.
+                int qn = 0;
+                const int nfull = sublen >> 10, nsteps = (sublen + 1023) >> 10;
+                auto load_step = [&](int w, int st, uint4 (&sv)[4]) {
+                    const uint4* rp = reinterpret_cast<const uint4*>(S + (size_t)w * ld + sub) + (st << 7) + lane;
+                    if (st < nfull) {
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) sv[q] = ldg_stream128(rp + q * 32);
-                } else {   // tail step; columns >= N of S hold -inf and their staged cost is 0: they never survive
+                        for (int q = 0; q < 4; ++q) sv[q] = ldg_stream128(rp + q * 32);
+                    } else {   // tail step; columns >= N of S hold -inf and their staged cost is 0: they never survive
+#pragma unroll
+                        for (int q = 0; q < 4; ++q) {
+                            sv[q] = make_uint4(0xfc00fc00u, 0xfc00fc00u, 0xfc00fc00u, 0xfc00fc00u);
+                            if ((st << 10) + q * 256 + lane * 8 < sublen) sv[q] = ldg_stream128(rp + q * 32);
+                        }
+                    }
+                };
+                auto flush = [&](int w) {
+                    const __half* srow = S + (size_t)w * ld + sub;
+                    const int wbase = sm.r_base[w], whb = sm.r_hbase[w], wnlo = sm.r_nlo[w], wshift = sm.r_shift[w];
+                    unsigned int* lw = seg_lists + (size_t)w * AUC_SEG_CAP;
+                    __syncwarp();
+                    for (int i0 = 0; i0 < qn; i0 += 32) {
+                        const int i = i0 + lane;
+                        bool live = i < qn;
+                        const int cc = live ? (int)wq[i] : 0;
+                        live = live && own_s[cc] != w;                               // owner entry: counted above
+                        int key = 0;
+                        if (live) key = (int)h2key(h2bits(__hsub(srow[cc], __ushort_as_half(cost_s[cc]))));
+                        const unsigned int m = __ballot_sync(0xffffffffu, live);
+                        if (m) {
+                            unsigned int slot0 = 0;
+                            if (lane == 0) slot0 = atomicAdd(&seg_cnt_s[w], (unsigned)__popc(m));
+                            slot0 = __shfl_sync(0xffffffffu, slot0, 0);
+                            const unsigned int slot = slot0 + __popc(m & lt);
+                            if (live && slot < AUC_SEG_CAP) lw[slot] = ((unsigned)cc << 16) | (unsigned)key;
+                        }
+                        if (live) {
+                            if (wshift == 0) {
+                                if (key >= whb) {
+                                    if (key - whb >= AUC_W - wnlo) atomicAdd(&sm.above[w], 1u);
+                                    else hist_add(sm.hist, w - h0, wnlo + key - whb);
+                                } else if (key >= wbase + wnlo) {
+                                    atomicAdd(&sm.gap[w], 1u);
+                                } else {
+                                    hist_add(sm.hist, w - h0, key - wbase);
+                                }
+                            } else {
+                                const int bin = (key - wbase) >> wshift;
+                                if (bin >= AUC_W) atomicAdd(&sm.above[w], 1u);
+                                else hist_add(sm.hist, w - h0, bin);
+                            }
+                        }
+                    }
+                    qn = 0;
+                    __syncwarp();
+                };
+                uint4 bufA[4], bufB[4];
+                int a = warp, st = 0;                                  // position in the active-row list, step in the row
+                int w = a < nact ? (int)acth[a] : 0;
+                if (a < nact) load_step(w, 0, bufA);
+                auto body = [&](uint4 (&cur)[4], uint4 (&nxt)[4]) {
+                    int an = a, wn = w, sn = st + 1;
+                    if (sn == nsteps) { an = a + AUC_NW; sn = 0; wn = an < nact ? (int)acth[an] : 0; }
+                    if (an < nact) load_step(wn, sn, nxt);
+                    // ---- filter: v = S - cost against the window's low edge ----
+                    const __half2 f2 = u2h2(sm.r_lo2[w]);
+                    const uint4* cp = reinterpret_cast<const uint4*>(cost_s) + (st << 7) + lane;
+                    unsigned int acc = 0;   // low half bit 4q+h: job 2h of load q survives; high half: job 2h+1
 #pragma unroll
                     for (int q = 0; q < 4; ++q) {
-                        sv[q] = make_uint4(0xfc00fc00u, 0xfc00fc00u, 0xfc00fc00u, 0xfc00fc00u);
-                        if ((st << 10) + q * 256 + lane * 8 < sublen) sv[q] = ldg_stream128(rp + q * 32);
-                    }
-                }
-            };
-            auto flush = [&](int w) {
-                const __half* srow = S + (size_t)w * ld + sub;
-                const int wbase = sm.r_base[w], whb = sm.r_hbase[w], wnlo = sm.r_nlo[w], wshift = sm.r_shift[w];
-                unsigned int* lw = seg_lists + (size_t)w * AUC_SEG_CAP;
-                __syncwarp();
-                for (int i0 = 0; i0 < qn; i0 += 32) {
-                    const int i = i0 + lane;
-                    bool live = i < qn;
-                    const int cc = live ? (int)wq[i] : 0;
-                    live = live && own_s[cc] != w;                               // owner entry: counted above
-                    int key = 0;
-                    if (live) key = (int)h2key(h2bits(__hsub(srow[cc], __ushort_as_half(cost_s[cc]))));
-                    const unsigned int m = __ballot_sync(0xffffffffu, live);
-                    if (m) {
-                        unsigned int slot0 = 0;
-                        if (lane == 0) slot0 = atomicAdd(&seg_cnt_s[w], (unsigned)__popc(m));
-                        slot0 = __shfl_sync(0xffffffffu, slot0, 0);
-                        const unsigned int slot = slot0 + __popc(m & lt);
-                        if (live && slot < AUC_SEG_CAP) lw[slot] = ((unsigned)cc << 16) | (unsigned)key;
-                    }
-                    if (live) {
-                        if (wshift == 0) {
-                            if (key >= whb) {
-                                if (key - whb >= AUC_W - wnlo) atomicAdd(&sm.above[w], 1u);
-                                else hist_add(sm.hist, w, wnlo + key - whb);
-                            } else if (key >= wbase + wnlo) {
-                                atomicAdd(&sm.gap[w], 1u);
-                            } else {
-                                hist_add(sm.hist, w, key - wbase);
-                            }
-                        } else {
-                            const int bin = (key - wbase) >> wshift;
-                            if (bin >= AUC_W) atomicAdd(&sm.above[w], 1u);
-                            else hist_add(sm.hist, w, bin);
+                        const uint4 cv = cp[q * 32];
+                        const unsigned int sw[4] = {cur[q].x, cur[q].y, cur[q].z, cur[q].w};
+                        const unsigned int cw[4] = {cv.x, cv.y, cv.z, cv.w};
+#pragma unroll
+                        for (int h = 0; h < 4; ++h) {
+                            const __half2 v2 = __hsub2(u2h2(sw[h]), u2h2(cw[h]));
+                            acc |= __hge2_mask(v2, f2) & ((1u << (4 * q + h)) | (1u << (16 + 4 * q + h)));
                         }
                     }
-                }
-                qn = 0;
-                __syncwarp();
-            };
-            uint4 bufA[4], bufB[4];
-            int a = warp, st = 0;                                  // position in the active-row list, step in the row
-            int w = a < nact ? (int)act[a] : 0;
-            if (a < nact) load_step(w, 0, bufA);
-            auto body = [&](uint4 (&cur)[4], uint4 (&nxt)[4]) {
-                int an = a, wn = w, sn = st + 1;
-                if (sn == nsteps) { an = a + AUC_NW; sn = 0; wn = an < nact ? (int)act[an] : 0; }
-                if (an < nact) load_step(wn, sn, nxt);
-                // ---- filter: v = S - cost against the window's low edge ----
-                const __half2 f2 = u2h2(sm.r_lo2[w]);
-                const uint4* cp = reinterpret_cast<const uint4*>(cost_s) + (st << 7) + lane;
-                unsigned int acc = 0;   // low half bit 4q+h: job 2h of load q survives; high half: job 2h+1
+                    // ---- push the survivors' job offsets ----
+                    const int mine = __popc(acc);
+                    int incl = mine;
 #pragma unroll
-                for (int q = 0; q < 4; ++q) {
-                    const uint4 cv = cp[q * 32];
-                    const unsigned int sw[4] = {cur[q].x, cur[q].y, cur[q].z, cur[q].w};
-                    const unsigned int cw[4] = {cv.x, cv.y, cv.z, cv.w};
-#pragma unroll
-                    for (int h = 0; h < 4; ++h) {
-                        const __half2 v2 = __hsub2(u2h2(sw[h]), u2h2(cw[h]));
-                        acc |= __hge2_mask(v2, f2) & ((1u << (4 * q + h)) | (1u << (16 + 4 * q + h)));
+                    for (int d = 1; d < 32; d <<= 1) {
+                        const int o = __shfl_up_sync(0xffffffffu, incl, d);
+                        if (lane >= d) incl += o;
                     }
-                }
-                // ---- push the survivors' job offsets ----
-                const int mine = __popc(acc);
-                int incl = mine;
-#pragma unroll
-                for (int d = 1; d < 32; d <<= 1) {
-                    const int o = __shfl_up_sync(0xffffffffu, incl, d);
-                    if (lane >= d) incl += o;
-                }
-                const int total = __shfl_sync(0xffffffffu, incl, 31);
-                if (total) {
-                    const int cbase = (st << 10) + lane * 8;
-                    if (qn + total > AUC_QCAP) flush(w);
-                    if (total <= AUC_QCAP) {
-                        int pos = qn + incl - mine;
-                        while (acc) {
-                            const int bpos = __ffs(acc) - 1;
-                            acc &= acc - 1;
-                            const int pq = bpos & 15;
-                            wq[pos++] = (unsigned short)(cbase + ((pq >> 2) << 8) + ((pq & 3) << 1) + (bpos >> 4));
-                        }
-                        qn += total;
-                    } else {
-                        // more than a queue's worth in one step (only with very wide windows): 4 per lane per round
-                        while (__any_sync(0xffffffffu, acc != 0)) {
-                            const int pc = __popc(acc);
-                            const int take = pc < 4 ? pc : 4;
-                            int in2 = take;
-#pragma unroll
-                            for (int d = 1; d < 32; d <<= 1) {
-                                const int o = __shfl_up_sync(0xffffffffu, in2, d);
-                                if (lane >= d) in2 += o;
-                            }
-                            int pos = in2 - take;
-                            for (int r = 0; r < take; ++r) {
+                    const int total = __shfl_sync(0xffffffffu, incl, 31);
+                    if (total) {
+                        const int cbase = (st << 10) + lane * 8;
+                        if (qn + total > AUC_QCAP) flush(w);
+                        if (total <= AUC_QCAP) {
+                            int pos = qn + incl - mine;
+                            while (acc) {
                                 const int bpos = __ffs(acc) - 1;
                                 acc &= acc - 1;
                                 const int pq = bpos & 15;
                                 wq[pos++] = (unsigned short)(cbase + ((pq >> 2) << 8) + ((pq & 3) << 1) + (bpos >> 4));
                             }
-                            qn = __shfl_sync(0xffffffffu, in2, 31);
-                            flush(w);
-                        }
-                    }
-                }
-                if (sn == 0 && qn) flush(w);                                     // the queue is per row
-                a = an;
-                w = wn;
-                st = sn;
-            };
-#if defined(RQK_HIST_PINGPONG)
-            while (a < nact) {                                                   // the two buffers used alternately
-                body(bufA, bufB);
-                if (a >= nact) break;
-                body(bufB, bufA);
-            }
-#else
-            while (a < nact) {
-                body(bufA, bufB);
+                            qn += total;
+                        } else {
+                            // more than a queue's worth in one step (only with very wide windows): 4 per lane per round
+                            while (__any_sync(0xffffffffu, acc != 0)) {
+                                const int pc = __popc(acc);
+                                const int take = pc < 4 ? pc : 4;
+                                int in2 = take;
 #pragma unroll
-                for (int q = 0; q < 4; ++q) bufA[q] = bufB[q];
-            }
-#endif
-        } else {
-            for (int a = warp; a < nact; a += AUC_NW) {
-                const int w = act[a];
-                const __half* srow = S + (size_t)w * ld + sub;
-                const int wbase = sm.r_base[w];
-                if (wbase > 0) {
-                    const int whb = sm.r_hbase[w], wnlo = sm.r_nlo[w], wshift = sm.r_shift[w];
-                    const __half lo = bits2h(key2h((unsigned)wbase));
-                    for (int c0 = 0; c0 < sublen; c0 += 32) {
-                        const int cc = c0 + lane;
-                        bool live = cc < sublen;
-                        if (live) live = __hge(__hsub(srow[cc], __ushort_as_half(cost_s[cc])), lo);
-                        if (__any_sync(0xffffffffu, live)) emit(w, srow, live, live ? cc : 0, wbase, whb, wnlo, wshift);
-                    }
-                } else {
-                    // cold row (all 65536 keys in 256 coarse bins): exact values, every element
-                    const int shift = sm.r_shift[w];
-                    for (int c0 = 0; c0 < sublen; c0 += 32) {
-                        const int cc = c0 + lane;
-                        const bool valid = cc < sublen;
-                        __half v = __ushort_as_half(0xfc00);
-                        if (valid) {
-                            const __half sx = srow[cc];
-                            v = (own_s[cc] == w) ? sx : __hsub(sx, __ushort_as_half(cost_s[cc]));
+                                for (int d = 1; d < 32; d <<= 1) {
+                                    const int o = __shfl_up_sync(0xffffffffu, in2, d);
+                                    if (lane >= d) in2 += o;
+                                }
+                                int pos = in2 - take;
+                                for (int r = 0; r < take; ++r) {
+                                    const int bpos = __ffs(acc) - 1;
+                                    acc &= acc - 1;
+                                    const int pq = bpos & 15;
+                                    wq[pos++] = (unsigned short)(cbase + ((pq >> 2) << 8) + ((pq & 3) << 1) + (bpos >> 4));
+                                }
+                                qn = __shfl_sync(0xffffffffu, in2, 31);
+                                flush(w);
+                            }
                         }
-                        const int bin = (int)h2key(h2bits(v)) >> shift;
-                        const bool hb = valid && bin < AUC_W;
-                        const bool ab = valid && bin >= AUC_W;
-                        unsigned int na = __popc(__ballot_sync(0xffffffffu, ab));
-                        if (lane == 0 && na) atomicAdd(&sm.above[w], na);
-                        unsigned int actm = __ballot_sync(0xffffffffu, hb);
-                        if (actm) {
-                            int lead = __ffs(actm) - 1;
-                            int lbin = __shfl_sync(0xffffffffu, bin, lead);
-                            unsigned int same = __ballot_sync(0xffffffffu, hb && bin == lbin);
-                            if (same == actm) {
-                                if (lane == lead) hist_add(sm.hist, w, lbin, __popc(actm));
-                            } else if (hb) {
-                                hist_add(sm.hist, w, bin);
+                    }
+                    if (sn == 0 && qn) flush(w);                                     // the queue is per row
+                    a = an;
+                    w = wn;
+                    st = sn;
+                };
+#if defined(RQK_HIST_PINGPONG)
+                while (a < nact) {                                                   // the two buffers used alternately
+                    body(bufA, bufB);
+                    if (a >= nact) break;
+                    body(bufB, bufA);
+                }
+#else
+                while (a < nact) {
+                    body(bufA, bufB);
+#pragma unroll
+                    for (int q = 0; q < 4; ++q) bufA[q] = bufB[q];
+                }
+#endif
+            } else {
+                for (int a = warp; a < nact; a += AUC_NW) {
+                    const int w = acth[a];
+                    const __half* srow = S + (size_t)w * ld + sub;
+                    const int wbase = sm.r_base[w];
+                    if (wbase > 0) {
+                        const int whb = sm.r_hbase[w], wnlo = sm.r_nlo[w], wshift = sm.r_shift[w];
+                        const __half lo = bits2h(key2h((unsigned)wbase));
+                        for (int c0 = 0; c0 < sublen; c0 += 32) {
+                            const int cc = c0 + lane;
+                            bool live = cc < sublen;
+                            if (live) live = __hge(__hsub(srow[cc], __ushort_as_half(cost_s[cc])), lo);
+                            if (__any_sync(0xffffffffu, live)) emit(w, srow, live, live ? cc : 0, wbase, whb, wnlo, wshift);
+                        }
+                    } else {
+                        // cold row (all 65536 keys in 256 coarse bins): exact values, every element
+                        const int shift = sm.r_shift[w];
+                        for (int c0 = 0; c0 < sublen; c0 += 32) {
+                            const int cc = c0 + lane;
+                            const bool valid = cc < sublen;
+                            __half v = __ushort_as_half(0xfc00);
+                            if (valid) {
+                                const __half sx = srow[cc];
+                                v = (own_s[cc] == w) ? sx : __hsub(sx, __ushort_as_half(cost_s[cc]));
+                            }
+                            const int bin = (int)h2key(h2bits(v)) >> shift;
+                            const bool hb = valid && bin < AUC_W;
+                            const bool ab = valid && bin >= AUC_W;
+                            unsigned int na = __popc(__ballot_sync(0xffffffffu, ab));
+                            if (lane == 0 && na) atomicAdd(&sm.above[w], na);
+                            unsigned int actm = __ballot_sync(0xffffffffu, hb);
+                            if (actm) {
+                                int lead = __ffs(actm) - 1;
+                                int lbin = __shfl_sync(0xffffffffu, bin, lead);
+                                unsigned int same = __ballot_sync(0xffffffffu, hb && bin == lbin);
+                                if (same == actm) {
+                                    if (lane == lead) hist_add(sm.hist, w - h0, lbin, __popc(actm));
+                                } else if (hb) {
+                                    hist_add(sm.hist, w - h0, bin);
+                                }
                             }
                         }
                     }
                 }
             }
+            __syncthreads();
+            if (tid >= h0 && tid < h0 + AUC_KH && tid < K && sm.r_shift[tid] != 0xff) {
+                const unsigned int c = seg_cnt_s[tid];
+                p.seg_cnt[(size_t)seg * K + tid] = c;
+                if (c > AUC_SEG_CAP) *p.list_ok = 0;
+            }
         }
-        __syncthreads();
-        if (tid < K && sm.r_shift[tid] != 0xff) {
-            const unsigned int c = seg_cnt_s[tid];
-            p.seg_cnt[(size_t)seg * K + tid] = c;
-            if (c > AUC_SEG_CAP) *p.list_ok = 0;
+
+        // ---- publish the half's histogram rows (active rows only) ----
+        // fused (single-GPU driver): plain stores into the per-CTA dump; auction_merge_resolve_kernel (one CTA per worker,
+        // next in the chain) sums them over the CTAs, resolves the worker's threshold and takes the tie prefix - no global
+        // atomics here, no serial resolve in a last CTA.  Step-by-step / sharded flows: the per-CTA dump (for the tie
+        // prefix) and a merge of the non-empty bins into the reduce block.
+        unsigned int* dump = reinterpret_cast<unsigned int*>(p.hist_cta + ((size_t)b * K + h0) * AUC_W);
+        for (int a = tid >> 7; a < nact; a += AUC_THREADS >> 7) {                // AUC_W / 2 = 128 words per row
+            const int i = ((int)acth[a] - h0) * (AUC_W / 2) + (tid & 127);
+            const unsigned int h = sm.hist[i];
+            dump[i] = h;
+            if (!fused) {
+                const int ig = h0 * (AUC_W / 2) + i;
+                if (h & 0xffffu) atomicAdd(&p.hist_g[2 * ig], h & 0xffffu);
+                if (h >> 16) atomicAdd(&p.hist_g[2 * ig + 1], h >> 16);
+            }
         }
+        ffh = 0;
     }
 
-    // ---- publish (active rows only) ----
-    unsigned int* dump = reinterpret_cast<unsigned int*>(p.hist_cta + (size_t)b * K * AUC_W);
-    if (fused) {
-        // single-GPU driver: plain stores of the CTA's histogram / above / gap counts.  auction_merge_resolve_kernel
-        // (one CTA per worker, next in the chain) sums them over the CTAs, resolves the worker's threshold and takes
-        // the tie prefix - no global atomics here, no serial resolve in a last CTA.
-        for (int a = tid >> 7; a < nact; a += AUC_THREADS >> 7) {
-            const int i = (int)act[a] * (AUC_W / 2) + (tid & 127);
-            dump[i] = sm.hist[i];
-        }
-        for (int a = tid; a < nact; a += AUC_THREADS) {
-            const int i = act[a];
+    const int nact_all = s_act_off[2];
+    for (int a = tid; a < nact_all; a += AUC_THREADS) {
+        const int i = act[a];
+        if (fused) {
             p.above_cta[(size_t)b * K + i] = sm.above[i];
             p.gap_cta[(size_t)b * K + i] = sm.gap[i];
+        } else {
+            if (sm.above[i]) atomicAdd(&p.above_g[i], sm.above[i]);
+            if (sm.gap[i]) atomicAdd(&p.gap_g[i], sm.gap[i]);
         }
-        return;
-    }
-    // step-by-step / sharded flows: per-CTA dump (for the tie prefix) + merge of non-empty bins into the reduce block
-    for (int a = tid >> 7; a < nact; a += AUC_THREADS >> 7) {                // AUC_W / 2 = 128 words per row
-        const int i = (int)act[a] * (AUC_W / 2) + (tid & 127);
-        const unsigned int h = sm.hist[i];
-        dump[i] = h;
-        if (h & 0xffffu) atomicAdd(&p.hist_g[2 * i], h & 0xffffu);
-        if (h >> 16) atomicAdd(&p.hist_g[2 * i + 1], h >> 16);
-    }
-    for (int a = tid; a < nact; a += AUC_THREADS) {
-        const int i = act[a];
-        if (sm.above[i]) atomicAdd(&p.above_g[i], sm.above[i]);
-        if (sm.gap[i]) atomicAdd(&p.gap_g[i], sm.gap[i]);
     }
 }
 
@@ -1681,8 +1709,6 @@ auction_bidlist_kernel(const __half* __restrict__ S, long long ld, long long N, 
     if (fused && auction_last_cta(p.ticket)) auction_resolve_body(p, n_global, K, n_global / K, MODE_BID);
 }
 
-static inline size_t auction_hist_smem(int K) { return K <= 128 ? HistSmem<128>::TOTAL : HistSmem<256>::TOTAL; }
-
 static inline size_t auction_pass_smem(int K, int J) {
     return (size_t)AUC_NBUF * K * J * 2 + (size_t)K * 16 + (size_t)J * 4 +
            (size_t)J * 4 + (size_t)K * 2 + (size_t)J + 64;
@@ -1692,7 +1718,7 @@ static inline size_t auction_pass_smem(int K, int J) {
 // sampled windows: instead of a coarse 3-pass radix descent from cold, estimate each worker's
 // threshold from a strided sample of its current values and open a fine window around the
 // estimate (+-4.5 sigma of the order statistic).  A wrong guess only costs a slide / coarse restart.
-// Grid = K CTAs x 1024 threads, 8192 samples (4096 left twice as many window misses at K = 256 on clustered data).
+// Grid = K CTAs x AUC_SAMPLE_THREADS threads, 8192 samples (4096 left twice as many window misses at K = 256 on clustered data).
 // ------------------------------------------------------------------------------------------
 constexpr int AUC_SAMPLE = AUC_SAMPLE_MAX;
 // Warp-parallel descending scan of a 256-bin histogram: the highest bin b with base + sum(hist[b..255]) >= need,
@@ -1731,7 +1757,7 @@ __device__ __forceinline__ void sample_select_bin(const unsigned int* hist, int 
 // Sharded jobs: every rank samples AUC_SAMPLE / world jobs of its shard (collect_out != null: write the keys
 // and return), the host all-gathers them, and every rank places identical windows from the union
 // (ext_keys != null: [ext_n / ext_cnt][K][ext_cnt] keys = every rank's gathered sample, N = global job count).
-__global__ void __launch_bounds__(1024, 1)
+__global__ void __launch_bounds__(AUC_SAMPLE_THREADS, 2)
 auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, int K, long long jpw, AuctionPtrs p,
                       unsigned short* __restrict__ collect_out, int collect_n,
                       const unsigned short* __restrict__ ext_keys, int ext_n, int ext_cnt, PeerCtx peers, int peer_par,
@@ -1755,46 +1781,51 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
     if (ext_keys || peers.world > 0) ns = ext_n;
     const __half eps = bits2h(st.eps_bits);
     {
-        constexpr int PER = AUC_SAMPLE / 1024;
-        __half c_r[PER], s_r[PER];
-        short o_r[PER];
-        unsigned short k_r[PER];
+        // a thread takes AUC_SAMPLE / AUC_SAMPLE_THREADS = 16 samples in two batches of 8: each batch issues all its
+        // loads first (one latency, not 8) within the 64 registers of two CTAs per SM
+        constexpr int PER = 8;
+        static_assert(AUC_SAMPLE % (PER * AUC_SAMPLE_THREADS) == 0, "whole batches");
         const long long nchunks = (ns + 15) / 16, cstride = N / (nchunks > 0 ? nchunks : 1);
+        for (int q0 = 0; q0 < AUC_SAMPLE / AUC_SAMPLE_THREADS; q0 += PER) {
+            __half c_r[PER], s_r[PER];
+            short o_r[PER];
+            unsigned short k_r[PER];
 #pragma unroll
-        for (int q = 0; q < PER; ++q) {                                        // all loads first: one latency, not PER
-            const int i = tid + q * 1024;
-            k_r[q] = 0;                                                        // padding sorts last
-            c_r[q] = s_r[q] = __ushort_as_half(0);
-            o_r[q] = -1;
-            if (ext_keys || peers.world > 0) {
-                if (i < ns) {
-                    if (peers.world > 0)      // part r = rank r's sample block, read through its peer mapping
-                        k_r[q] = __ldcv(peer_sample(peers, i / ext_cnt, K, peer_par) + (size_t)w * ext_cnt + (i % ext_cnt));
-                    else
-                        k_r[q] = ext_keys[((size_t)(i / ext_cnt) * K + w) * ext_cnt + (i % ext_cnt)];   // [part][K][ext_cnt]
+            for (int q = 0; q < PER; ++q) {
+                const int i = tid + (q0 + q) * AUC_SAMPLE_THREADS;
+                k_r[q] = 0;                                                    // padding sorts last
+                c_r[q] = s_r[q] = __ushort_as_half(0);
+                o_r[q] = -1;
+                if (ext_keys || peers.world > 0) {
+                    if (i < ns) {
+                        if (peers.world > 0)      // part r = rank r's sample block, read through its peer mapping
+                            k_r[q] = __ldcv(peer_sample(peers, i / ext_cnt, K, peer_par) + (size_t)w * ext_cnt + (i % ext_cnt));
+                        else
+                            k_r[q] = ext_keys[((size_t)(i / ext_cnt) * K + w) * ext_cnt + (i % ext_cnt)];   // [part][K][ext_cnt]
+                    }
+                } else if (i < ns) {
+                    // 16 consecutive jobs = one 32-byte sector of the row; chunks evenly strided over the jobs
+                    long long col = cstride * (i >> 4) + (i & 15);
+                    if (col >= N) col = N - 1;
+                    c_r[q] = p.cost[col];
+                    o_r[q] = p.owner[col];
+                    s_r[q] = S[(size_t)w * ld + col];
                 }
-            } else if (i < ns) {
-                // 16 consecutive jobs = one 32-byte sector of the row; chunks evenly strided over the jobs
-                long long col = cstride * (i >> 4) + (i & 15);
-                if (col >= N) col = N - 1;
-                c_r[q] = p.cost[col];
-                o_r[q] = p.owner[col];
-                s_r[q] = S[(size_t)w * ld + col];
             }
-        }
 #pragma unroll
-        for (int q = 0; q < PER; ++q) {
-            const int i = tid + q * 1024;
-            unsigned short key = k_r[q];
-            if (!ext_keys && peers.world == 0 && i < ns) {
-                __half c = c_r[q];
-                if (st.ff_pending > 0 && o_r[q] >= 0)
-                    for (int r = 0; r < st.ff_pending; ++r) c = __hadd(c, eps);
-                const __half v = (o_r[q] == w) ? s_r[q] : __hsub(s_r[q], c);
-                key = (unsigned short)h2key(h2bits(v));
+            for (int q = 0; q < PER; ++q) {
+                const int i = tid + (q0 + q) * AUC_SAMPLE_THREADS;
+                unsigned short key = k_r[q];
+                if (!ext_keys && peers.world == 0 && i < ns) {
+                    __half c = c_r[q];
+                    if (st.ff_pending > 0 && o_r[q] >= 0)
+                        for (int r = 0; r < st.ff_pending; ++r) c = __hadd(c, eps);
+                    const __half v = (o_r[q] == w) ? s_r[q] : __hsub(s_r[q], c);
+                    key = (unsigned short)h2key(h2bits(v));
+                }
+                keys[i] = key;
+                if (collect_out && i < collect_n) collect_out[(size_t)w * collect_n + i] = key;
             }
-            keys[i] = key;
-            if (collect_out && i < collect_n) collect_out[(size_t)w * collect_n + i] = key;
         }
     }
     if (collect_out) return;
@@ -1816,14 +1847,14 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
             if (tid < 256) shist[tid] = 0;
             if (tid == 0) s_cnt = 0;
             __syncthreads();
-            for (int i = tid; i < AUC_SAMPLE; i += 1024) atomicAdd(&shist[keys[i] >> 8], 1u);
+            for (int i = tid; i < AUC_SAMPLE; i += AUC_SAMPLE_THREADS) atomicAdd(&shist[keys[i] >> 8], 1u);
             __syncthreads();
             if (tid < 32) sample_select_bin(shist, 0, need_n, &s_b1, &s_above1);
             __syncthreads();
             const int b1 = s_b1;
             if (tid < 256) shist[tid] = 0;
             __syncthreads();
-            for (int i = tid; i < AUC_SAMPLE; i += 1024)
+            for (int i = tid; i < AUC_SAMPLE; i += AUC_SAMPLE_THREADS)
                 if ((keys[i] >> 8) == b1) atomicAdd(&shist[keys[i] & 255], 1u);
             __syncthreads();
             if (tid < 32) {
@@ -1833,7 +1864,7 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
             }
             __syncthreads();
             const int vlo = s_vlo;
-            for (int i = tid; i < AUC_SAMPLE; i += 1024) {
+            for (int i = tid; i < AUC_SAMPLE; i += AUC_SAMPLE_THREADS) {
                 const unsigned short kk = keys[i];
                 if ((int)kk >= vlo) {
                     const int slot = atomicAdd(&s_cnt, 1);
@@ -1844,7 +1875,7 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
             const int cnt = s_cnt;
             if (cnt <= 1024) {
                 need_full_sort = false;
-                for (int i = tid; i < cnt; i += 1024) {
+                for (int i = tid; i < cnt; i += AUC_SAMPLE_THREADS) {
                     const unsigned short kk = top[i];
                     int rank = 0;
                     for (int j = 0; j < cnt; ++j) {
@@ -1854,7 +1885,7 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
                     sorted[rank] = kk;
                 }
                 __syncthreads();
-                for (int i = tid; i < cnt; i += 1024) keys[i] = sorted[i];   // ranks 0 .. cnt-1 (>= r_lo) are exact
+                for (int i = tid; i < cnt; i += AUC_SAMPLE_THREADS) keys[i] = sorted[i];   // ranks 0 .. cnt-1 (>= r_lo) are exact
                 __syncthreads();
             }
         }
@@ -1863,7 +1894,7 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
         // bitonic sort, descending
         for (int k = 2; k <= AUC_SAMPLE; k <<= 1) {
             for (int j = k >> 1; j > 0; j >>= 1) {
-                for (int i = tid; i < AUC_SAMPLE; i += 1024) {
+                for (int i = tid; i < AUC_SAMPLE; i += AUC_SAMPLE_THREADS) {
                     const int ixj = i ^ j;
                     if (ixj > i) {
                         const unsigned short a = keys[i], b2 = keys[ixj];
@@ -2557,18 +2588,17 @@ static int auction_launch(const AuctionArgs& a, const void* scores_t, int64_t ld
     }
     const int spc = auction_spc(n, k);
     if (which & 1)
-        RQK_CUDA_OK(launch_round_kernel(auction_sample_kernel, (unsigned)k, 1024u, 0, stream, pdl, (const __half*)scores_t,
+        RQK_CUDA_OK(launch_round_kernel(auction_sample_kernel, (unsigned)k, (unsigned)AUC_SAMPLE_THREADS, 0, stream, pdl, (const __half*)scores_t,
                                         (long long)ld, (long long)n, (int)k, (long long)(n_global / k), a.p,
                                         (unsigned short*)nullptr, 0, (const unsigned short*)nullptr, 0, 1, PeerCtx{}, 0, -1));
     if (which & 2) {
-        static bool hs_set[RQK_MAX_DEVICES][2] = {};
-        const size_t hs = auction_hist_smem(k);
-        auto hkern = (k <= 128) ? auction_hist_kernel<128> : auction_hist_kernel<256>;
-        if (!hs_set[devi][k <= 128 ? 0 : 1]) {
-            RQK_CUDA_OK(cudaFuncSetAttribute(hkern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hs));
-            hs_set[devi][k <= 128 ? 0 : 1] = true;
+        static bool hs_set[RQK_MAX_DEVICES] = {};
+        const size_t hs = HistSmem::TOTAL;
+        if (!hs_set[devi]) {
+            RQK_CUDA_OK(cudaFuncSetAttribute(auction_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hs));
+            hs_set[devi] = true;
         }
-        RQK_CUDA_OK(launch_round_kernel(hkern, (unsigned)a.G, (unsigned)AUC_THREADS, hs, stream, pdl,
+        RQK_CUDA_OK(launch_round_kernel(auction_hist_kernel, (unsigned)a.G, (unsigned)AUC_THREADS, hs, stream, pdl,
                                         (const __half*)scores_t, (long long)ld, (long long)n, (int)k, a.J, spc, a.p,
                                         (long long)n_global, fused));
     }
@@ -2677,7 +2707,7 @@ int rqk_auction_sample_collect(const void* scores_t, int64_t ld, int64_t n, int3
     int rc = auction_prepare(n, ld, k, workspace, workspace_bytes, &a, "rqk_auction_sample_collect");
     if (rc) return rc;
     if (!scores_t || !out || count < 1 || count > AUC_SAMPLE) return fail(RQK_ERR_ARG, "rqk_auction_sample_collect: bad argument%s");
-    auction_sample_kernel<<<k, 1024, 0, (cudaStream_t)stream_>>>((const __half*)scores_t, ld, n, k, n_global / k, a.p,
+    auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, (cudaStream_t)stream_>>>((const __half*)scores_t, ld, n, k, n_global / k, a.p,
                                                                   (unsigned short*)out, count, nullptr, 0, 1, PeerCtx{}, 0, -1);
     RQK_LAUNCH_OK();
     return 0;
@@ -2693,7 +2723,7 @@ int rqk_auction_sample_window(int64_t n, int64_t ld, int32_t k, int64_t n_global
     if (rc) return rc;
     if (!keys || count < 1 || parts < 1 || (int64_t)count * parts > AUC_SAMPLE)
         return fail(RQK_ERR_ARG, "rqk_auction_sample_window: bad argument%s");
-    auction_sample_kernel<<<k, 1024, 0, (cudaStream_t)stream_>>>(nullptr, ld, n_global, k, n_global / k, a.p, nullptr, 0,
+    auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, (cudaStream_t)stream_>>>(nullptr, ld, n_global, k, n_global / k, a.p, nullptr, 0,
                                                                   (const unsigned short*)keys, count * parts, count, PeerCtx{}, 0, -1);
     RQK_LAUNCH_OK();
     return 0;
@@ -2747,10 +2777,10 @@ int rqk_auction_peer_sample(const void* scores_t, int64_t ld, int64_t n, int32_t
     if (!scores_t || count < 1 || (int64_t)count * world > AUC_SAMPLE) return fail(RQK_ERR_ARG, "rqk_auction_peer_sample: bad argument%s");
     cudaStream_t stream = (cudaStream_t)stream_;
     unsigned short* mine = reinterpret_cast<unsigned short*>(c.buf[rank] + peer_sample_off(k)) + (size_t)(seq & 1) * k * AUC_SAMPLE_MAX;
-    auction_sample_kernel<<<k, 1024, 0, stream>>>((const __half*)scores_t, ld, n, k, n_global / k, a.p, mine, count, nullptr, 0, 1,
+    auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, stream>>>((const __half*)scores_t, ld, n, k, n_global / k, a.p, mine, count, nullptr, 0, 1,
                                                   PeerCtx{}, 0, -1);
     auction_peer_barrier_kernel<<<1, 32, 0, stream>>>(a.p, c, 0, seq);
-    auction_sample_kernel<<<k, 1024, 0, stream>>>(nullptr, ld, n_global, k, n_global / k, a.p, nullptr, 0, nullptr, count * world, count,
+    auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, stream>>>(nullptr, ld, n_global, k, n_global / k, a.p, nullptr, 0, nullptr, count * world, count,
                                                   c, seq & 1, -1);
     RQK_LAUNCH_OK();
     return 0;
@@ -2781,7 +2811,7 @@ int rqk_auction_peer_round(const void* scores_t, int64_t ld, int64_t n, int32_t 
     RQK_CUDA_OK(launch_round_kernel(auction_peer_bid_collect_kernel, (unsigned)k, 1024u, 0, stream, pdl, (const __half*)scores_t,
                                     (long long)ld, (long long)n, (int)k, (long long)n_global, a.p, (int)count, c, (int)seq0,
                                     (int)(seq0 + 1)));
-    RQK_CUDA_OK(launch_round_kernel(auction_sample_kernel, (unsigned)k, 1024u, 0, stream, pdl, (const __half*)nullptr, (long long)ld,
+    RQK_CUDA_OK(launch_round_kernel(auction_sample_kernel, (unsigned)k, (unsigned)AUC_SAMPLE_THREADS, 0, stream, pdl, (const __half*)nullptr, (long long)ld,
                                     (long long)n_global, (int)k, (long long)(n_global / k), a.p, (unsigned short*)nullptr, 0,
                                     (const unsigned short*)nullptr, (int)(count * world), (int)count, c, (int)((seq0 + 1) & 1),
                                     (int)(seq0 + 1)));
