@@ -45,10 +45,7 @@ SIGNATURES = {
     "rqk_auction_sample_window": (ctypes.c_int, [c_i64, c_i64, c_i32, c_i64, c_p, c_i32, c_i32, c_p, c_sz, c_p]),
     "rqk_auction_resolve": (ctypes.c_int, [c_i64, c_i64, c_i32, c_i64, c_i32, c_p, c_sz, c_p]),
     "rqk_auction_peer_bytes": (c_sz, [c_i32]),
-    "rqk_auction_peer_hist_bytes": (c_sz, [c_i32]),
-    "rqk_auction_peer_sample": (ctypes.c_int, [c_p, c_i64, c_i64, c_i32, c_i64, c_i32, c_p, c_i32, c_i32, c_i32, c_p, c_sz, c_p]),
     "rqk_auction_peer_round": (ctypes.c_int, [c_p, c_i64, c_i64, c_i32, c_i64, c_i32, c_p, c_i32, c_i32, c_i32, c_p, c_sz, c_p]),
-    "rqk_auction_peer_resolve": (ctypes.c_int, [c_i64, c_i64, c_i32, c_i64, c_i32, c_p, c_i32, c_i32, c_i32, c_p, c_sz, c_p]),
     "rqk_auction_tie_offset": (ctypes.c_int, [c_i64, c_i64, c_i32, c_p, c_i32, c_p, c_sz, c_p]),
     "rqk_auction_poll": (ctypes.c_int, [c_i64, c_i64, c_i32, c_p, c_sz, ctypes.POINTER(AuctionInfo), c_p]),
     "rqk_auction_finalize": (ctypes.c_int, [c_i64, c_i64, c_i32, c_p, c_sz, c_p, c_p]),

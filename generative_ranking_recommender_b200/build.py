@@ -29,11 +29,10 @@ def build(force: bool = False, verbose: bool = False) -> str:
     objs = []
     procs = []
     os.makedirs(os.path.join(HERE, "build"), exist_ok=True)
-    extra = os.environ.get("RQK_NVCC_EXTRA", "").split()      # experiments: -DNAME=value switches of a kernel variant
     for src in SOURCES:
         obj = os.path.join(HERE, "build", src.replace(".cu", ".o"))
         objs.append(obj)
-        cmd = [nvcc, *NVCC_FLAGS, *extra, "-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [nvcc, *NVCC_FLAGS, "-c", os.path.join(CSRC, src), "-o", obj]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
         procs.append((src, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True)))

@@ -12,26 +12,32 @@
 //          streams through shared memory, and bids are reduced to (highest bid, first highest
 //          bidder) per job on the fly.
 //
-// A ROUND of the reference is two streaming passes over S (2*K bytes per job each):
-//   HIST pass  (auction_hist_kernel) each worker's threshold T_w, the (N/K+1)-th largest value (:66), by an
-//            exact 16-bit radix select.  A strided 4096-job sample of the worker's current values brackets the
-//            threshold's rank (+-4.5 sigma of the order statistic, capped by the previous threshold: costs only
-//            grow, so thresholds only sink); 256 one-key bins are laid over that bracket (split in two runs
-//            around the widest sampled hole if it is wider than 256 keys) plus "above" / "gap" counters.
-//            Warps stream row segments straight from global memory (16-byte loads, four in flight per lane):
-//            per 8 jobs 1 LDG.128 + 1 LDS.128 + 4 HSUB2 + 4 HSET2 + 4 LOP3; the ~1.5 % survivors (values at or
-//            above the bracket's low edge) are kept as register bitmasks and histogrammed afterwards (16-bit
-//            packed shared-memory counters).  A 1-CTA resolve kernel turns the merged histograms into exact
-//            thresholds (hit -> exact; miss -> slide / refine / coarse restart); a K-CTA kernel prefix-sums
-//            per-CTA tie counts so the canonical tie rule is global.
-//   BID pass   (auction_pass_kernel) tiles of all K workers x 128 (K<=128) or 64 jobs in shared memory through a
-//            3-deep bulk-copy (UBLKCP + mbarrier) ring.  A warp owns a worker row of the tile, so ties are met
-//            in job order.  The sweep is a half2 FILTER: v = S - cost (ownership ignored: the owner's true value
-//            S is only larger) against T_w; survivors (~0.8 %) are register bitmasks and become bids
-//            ((v - T_w) + eps, :76); ties at T_w are taken lowest job index first up to the worker's quota.
-//            The one owner entry of every job is handled by the job's column thread (retain hack :86-87,
-//            counter>1000 fallback :88-89).  The column max with first-argmax (:104) is an atomicMax on
-//            (bid << 16 | ~worker) in shared memory; then cost/owner update (:118-123).
+// A ROUND of the reference finds each worker's threshold T_w, the (N/K+1)-th largest value (:66), and then bids.
+// Here that is a chain of kernels; a device-side state machine decides what the round needs, and a kernel whose turn
+// it is not returns at once.
+//   window sampling  (auction_sample_kernel, K CTAs) a strided 8192-job sample of each worker's current values
+//            brackets the threshold's rank (+-4.5 sigma of the order statistic, capped by the previous threshold:
+//            costs only grow, so thresholds only sink); 256 one-key bins are laid over that bracket (split in two
+//            runs around the widest sampled hole if it is wider than 256 keys, coarser bins if even that does not
+//            fit) plus "above" / "gap" counters.
+//   HIST pass  (auction_hist_kernel, G CTAs) the exact 16-bit radix select over that window.  Warps stream row
+//            segments straight from global memory (16-byte loads, four in flight per lane): per 8 jobs 1 LDG.128
+//            + 1 LDS.128 + 4 HSUB2 + 4 HSET2 + 4 LOP3.  The ~1.5 % survivors (values at or above the window's low
+//            edge) are histogrammed in 16-bit packed shared-memory counters and appended to the survivor list of
+//            their (4096-job sub-range, worker).  The histograms are dumped per CTA (or, in the step-by-step flow,
+//            merged with atomics into the reduce block).
+//   merge + resolve  (auction_merge_resolve_kernel, one CTA per worker) sums the worker's dumps, turns them into an
+//            exact threshold (hit -> exact; miss -> slide / refine / coarse restart; a coarse bin is refined from
+//            the survivor lists) and prefix-sums the per-CTA tie counts so the canonical tie rule is global.
+//   bid-list replay  (auction_bidlist_kernel, G CTAs) the bidding round from the survivor lists, without reading S
+//            again: bids ((v - T_w) + eps, :76), ties at T_w taken lowest job index first up to the worker's quota,
+//            retain hack (:86-87) and counter>1000 fallback (:88-89) per job, column max with first-argmax (:104),
+//            cost / owner update (:118-123).
+//   S-scanning fallback  (auction_pass_kernel, after a survivor-list overflow) the same bidding round from tiles of
+//            all K workers x 128 (K<=128) or 64 jobs, bulk-copied into shared memory through a 3-deep ring.
+// In the single-GPU driver the last CTA of the bidding kernel runs the resolve step (termination, frozen detection,
+// next state).  With the jobs sharded over GPUs the same kernels run on every rank's shard, and the sums over ranks
+// happen either inside the kernels over peer memory (rqk_auction_peer_round) or through NCCL between step functions.
 //
 // Exact fast-forward.  With N % K != 0 the reference cannot terminate before its counter>1000
 // fallback and runs 1002 rounds (SURVEY.md F4).  But once a round's fresh bids all land on jobs
@@ -280,10 +286,10 @@ __global__ void auction_init_kernel(AuctionPtrs p, long long ld, int K, const un
 // the host: torch symmetric memory); kernels read the other ranks' blocks directly and synchronise
 // with monotonically increasing sequence flags, so that the collective a round needs (sum of the
 // threshold histograms, rank-major tie counts, the two bid counters, the window samples) is part of
-// the resolve / sampling kernel instead of a library call between two kernels.
+// the round's kernels instead of a library call between two kernels.
 //   flags  int32 [3 kinds][8 ranks]   flags[kind][r] = last sequence number rank r has published
 //   tail   int32 [2 parities][2]      jobs with a bidder, frozen-state violations of the local BID round
-//   hist   int32 [2 parities][RB]     local reduce block (RB = K*256 + 2K + 2)
+//   hist   int32 [2 parities][RB]     local histogram rows [K][256], above [K], gap [K] (RB >= K*256 + 2K)
 //   sample uint16[2 parities][K][cnt] local window samples
 // Blocks are double-buffered by the parity of the sequence number: a rank can only be two exchanges
 // ahead of a peer that still reads its block, never in the same parity.
@@ -311,7 +317,7 @@ __device__ __forceinline__ const unsigned short* peer_sample(const PeerCtx& c, i
 // All threads of the CTA call this after their stores to the local exchange block.  Returns false on a timeout
 // (a peer that never arrives: 4 s), which the caller turns into an error state instead of a hang.
 // `signal` = false: wait only (another CTA of the grid publishes this rank's arrival).
-__device__ bool peer_barrier(const PeerCtx& c, int kind, int seq, bool signal = true) {
+__device__ bool peer_barrier(const PeerCtx& c, int kind, int seq, bool signal) {
     __shared__ int s_ok;
     __threadfence_system();
     __syncthreads();
@@ -584,100 +590,6 @@ __device__ __forceinline__ bool auction_last_cta(unsigned int* ticket) {
     __syncthreads();
     if (s_last) __threadfence();
     return s_last != 0;
-}
-
-
-// Resolve step of a sharded job with the rank exchange inside (1 CTA per rank).  expect = MODE_HIST: publish
-// the local reduce block, wait for the peers, sum theirs into it, resolve, and derive this rank's tie offsets
-// from the peers' LOCAL histograms at the resolved threshold bins; expect = MODE_BID: the same for the two bid
-// counters.  Every rank runs the identical state machine, so all take the same early exits.
-__global__ void __launch_bounds__(1024, 1)
-auction_resolve_peer_kernel(AuctionPtrs p, long long N, int K, long long jpw, int expect, PeerCtx peers, int seq) {
-    const int mode = p.st->mode;
-    if (mode == MODE_DONE || mode != expect) return;
-    const int tid = threadIdx.x, NT = blockDim.x, par = seq & 1;
-    const int RB = K * AUC_W + 2 * K + 2;
-    if (expect == MODE_HIST) {
-        unsigned int* mine = peer_hist(peers, peers.rank, K, par);
-        for (int i0 = tid; i0 < RB; i0 += 8 * NT) {            // 8 independent loads in flight per thread
-            unsigned int v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u) v[u] = (i0 + u * NT < RB) ? __ldcg(p.hist_g + i0 + u * NT) : 0u;
-#pragma unroll
-            for (int u = 0; u < 8; ++u) if (i0 + u * NT < RB) mine[i0 + u * NT] = v[u];
-        }
-        if (!peer_barrier(peers, 1, seq)) { if (tid == 0) { p.st->error = 1; p.st->mode = MODE_DONE; p.st->done = 1; } return; }
-        // a peer load costs 2-3 us of NVLink latency: keep 4 words x (world - 1) peers in flight per thread
-        for (int i0 = tid; i0 < RB; i0 += 4 * NT) {
-            unsigned int acc[4] = {0u, 0u, 0u, 0u};
-#pragma unroll
-            for (int r = 0; r < PEER_MAX; ++r) {
-                if (r >= peers.world || r == peers.rank) continue;
-                const unsigned int* theirs = peer_hist(peers, r, K, par);
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    const int i = i0 + u * NT;
-                    if (i < RB) acc[u] += __ldcv(theirs + i);
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int i = i0 + u * NT;
-                if (i < RB) p.hist_g[i] += acc[u];
-            }
-        }
-        __syncthreads();
-        const int this_pass = p.st->passes;
-        __syncthreads();
-        auction_resolve_body(p, N, K, jpw, expect);
-        __syncthreads();
-        {
-            // rank-major tie offsets of the workers THIS pass resolved (a partial pass after a window miss streams
-            // only the workers that missed; the peers' blocks of this exchange hold nothing for the others)
-            for (int w = tid; w < K; w += NT) {
-                if (p.res_pass[w] != this_pass || p.tkey[w] < 0) continue;
-                const int base = p.win_base[w], hbase = p.win_hbase[w], nlo = p.win_nlo[w], tk = p.tkey[w];
-                const int bin = tk >= hbase ? nlo + tk - hbase : tk - base;
-                unsigned int part[PEER_MAX];
-#pragma unroll
-                for (int r = 0; r < PEER_MAX; ++r)                // all lower ranks' loads in flight together
-                    part[r] = (r < peers.rank) ? __ldcv(peer_hist(peers, r, K, par) + (size_t)w * AUC_W + bin) : 0u;
-                unsigned int off = 0;
-#pragma unroll
-                for (int r = 0; r < PEER_MAX; ++r) off += part[r];
-                p.rank_off[w] = off;
-            }
-        }
-    } else {
-        if (tid == 0) {
-            int* mine = peer_tail(peers, peers.rank, par);
-            mine[0] = (int)*p.n_with;
-            mine[1] = (int)*p.n_viol;
-        }
-        if (!peer_barrier(peers, 2, seq)) { if (tid == 0) { p.st->error = 1; p.st->mode = MODE_DONE; p.st->done = 1; } return; }
-        if (tid < 32) {                                        // one lane per rank: the peer loads overlap
-            unsigned int a = 0, b = 0;
-            if (tid < peers.world) {
-                const int* t = peer_tail(peers, tid, par);
-                a = (unsigned int)__ldcv(t);
-                b = (unsigned int)__ldcv(t + 1);
-            }
-#pragma unroll
-            for (int d = 16; d; d >>= 1) {
-                a += __shfl_xor_sync(0xffffffffu, a, d);
-                b += __shfl_xor_sync(0xffffffffu, b, d);
-            }
-            if (tid == 0) { *p.n_with = a; *p.n_viol = b; }
-        }
-        __syncthreads();
-        auction_resolve_body(p, N, K, jpw, expect);
-    }
-}
-
-// Between the local sample collection and the window placement: every rank's samples are in place.
-__global__ void auction_peer_barrier_kernel(AuctionPtrs p, PeerCtx peers, int kind, int seq) {
-    if (p.st->mode != MODE_HIST || !p.st->need_sample) return;
-    if (!peer_barrier(peers, kind, seq) && threadIdx.x == 0) { p.st->error = 1; p.st->mode = MODE_DONE; p.st->done = 1; }
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1058,13 +970,8 @@ auction_pass_kernel(const __half* __restrict__ S, long long ld, long long N, int
 constexpr int HS_SUB = AUC_SUB;   // jobs staged (cost, owner) per sub-range
 __device__ __forceinline__ uint4 ldg_stream128(const void* ptr) {
     uint4 r;
-#if defined(RQK_HIST_NOALLOC)
-    asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0, %1, %2, %3}, [%4];"
-                 : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(ptr));
-#else
     asm volatile("ld.global.nc.v4.u32 {%0, %1, %2, %3}, [%4];"
                  : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(ptr));
-#endif
     return r;
 }
 
@@ -1381,19 +1288,11 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
                     w = wn;
                     st = sn;
                 };
-#if defined(RQK_HIST_PINGPONG)
-                while (a < nact) {                                                   // the two buffers used alternately
-                    body(bufA, bufB);
-                    if (a >= nact) break;
-                    body(bufB, bufA);
-                }
-#else
                 while (a < nact) {
                     body(bufA, bufB);
 #pragma unroll
                     for (int q = 0; q < 4; ++q) bufA[q] = bufB[q];
                 }
-#endif
             } else {
                 for (int a = warp; a < nact; a += AUC_NW) {
                     const int w = acth[a];
@@ -1757,21 +1656,21 @@ __device__ __forceinline__ void sample_select_bin(const unsigned int* hist, int 
 // Sharded jobs: every rank samples AUC_SAMPLE / world jobs of its shard (collect_out != null: write the keys
 // and return), the host all-gathers them, and every rank places identical windows from the union
 // (ext_keys != null: [ext_n / ext_cnt][K][ext_cnt] keys = every rank's gathered sample, N = global job count).
+// peers.world > 0: the parts are the ranks' exchange blocks instead (parity of peer_seq), after a flag barrier.
 __global__ void __launch_bounds__(AUC_SAMPLE_THREADS, 2)
 auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, int K, long long jpw, AuctionPtrs p,
                       unsigned short* __restrict__ collect_out, int collect_n,
-                      const unsigned short* __restrict__ ext_keys, int ext_n, int ext_cnt, PeerCtx peers, int peer_par,
-                      int barrier_seq) {
+                      const unsigned short* __restrict__ ext_keys, int ext_n, int ext_cnt, PeerCtx peers, int peer_seq) {
     pdl_launch_dependents();
     pdl_wait();
     const AuctionState st = *p.st;
     if (st.mode != MODE_HIST || !st.need_sample) return;
     __shared__ unsigned short keys[AUC_SAMPLE];
     const int w = blockIdx.x, tid = threadIdx.x;
-    if (peers.world > 0 && barrier_seq >= 0) {
+    if (peers.world > 0) {
         // every rank's samples are in its exchange block once the kernel before this one has completed (which the
         // wait above guarantees): CTA 0 publishes this rank's arrival, every CTA waits for all ranks
-        if (!peer_barrier(peers, 0, barrier_seq, blockIdx.x == 0)) {
+        if (!peer_barrier(peers, 0, peer_seq, blockIdx.x == 0)) {
             if (tid == 0) { p.st->error = 1; p.st->mode = MODE_DONE; p.st->done = 1; }
             return;
         }
@@ -1799,7 +1698,7 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
                 if (ext_keys || peers.world > 0) {
                     if (i < ns) {
                         if (peers.world > 0)      // part r = rank r's sample block, read through its peer mapping
-                            k_r[q] = __ldcv(peer_sample(peers, i / ext_cnt, K, peer_par) + (size_t)w * ext_cnt + (i % ext_cnt));
+                            k_r[q] = __ldcv(peer_sample(peers, i / ext_cnt, K, peer_seq & 1) + (size_t)w * ext_cnt + (i % ext_cnt));
                         else
                             k_r[q] = ext_keys[((size_t)(i / ext_cnt) * K + w) * ext_cnt + (i % ext_cnt)];   // [part][K][ext_cnt]
                     }
@@ -1965,17 +1864,18 @@ auction_sample_kernel(const __half* __restrict__ S, long long ld, long long N, i
 // ------------------------------------------------------------------------------------------
 // Sharded jobs, whole-round protocol (rqk_auction_peer_round): seven launches per round, chained with programmatic
 // dependent launch, three flag barriers that sit INSIDE kernels which have work of their own:
-//   1. auction_peer_bid_collect_kernel  (K CTAs)   counters of the previous round's bids exchanged and resolved
-//                                                  (every CTA derives the next state from the summed counters, the
-//                                                  LAST CTA applies it), then the local window samples
-//   2. auction_sample_kernel            (K CTAs)   sample barrier, windows from the union of all ranks' samples
-//   3. auction_hist_kernel              (G CTAs)   merges straight into this rank's exchange block
-//   4. auction_peer_exchange_kernel     (16 CTAs)  histogram barrier, every CTA sums a slice over the ranks (one NVLink
-//                                                  round trip), last CTA resolves + rank-major tie offsets
-//   5. tie prefix, 6. bid-list replay, 7. S-scanning fallback (returns at once unless a list overflowed)
+//   1. auction_peer_bid_collect_kernel      (K CTAs)  counters of the previous round's bids exchanged and resolved
+//                                                     (every CTA derives the next state from the summed counters, the
+//                                                     LAST CTA applies it), then the local window samples
+//   2. auction_sample_kernel                (K CTAs)  sample barrier, windows from the union of all ranks' samples
+//   3. auction_hist_kernel                  (G CTAs)  dumps its histograms per CTA, as in the single-GPU driver
+//   4. auction_peer_publish_kernel          (K CTAs)  CTA w sums worker w's dumps into this rank's exchange block; the
+//                                                     last CTA signals the peers (histogram barrier)
+//   5. auction_peer_resolve_workers_kernel  (K CTAs)  CTA w waits for the peers, sums worker w's row over the ranks,
+//                                                     resolves it and takes its rank-major tie prefix
+//   6. auction_bidlist_kernel               (G CTAs)  bid-list replay
+//   7. auction_pass_kernel                  (G CTAs)  S-scanning fallback (returns at once unless a list overflowed)
 // ------------------------------------------------------------------------------------------
-constexpr int PEER_XCH_CTAS = 16;
-
 __global__ void __launch_bounds__(1024, 1)
 auction_peer_bid_collect_kernel(const __half* __restrict__ S, long long ld, long long N, int K, long long n_global,
                                 AuctionPtrs p, int count, PeerCtx peers, int seq_bid, int seq_sample) {
@@ -2057,56 +1957,8 @@ auction_peer_bid_collect_kernel(const __half* __restrict__ S, long long ld, long
     }
 }
 
-// HIST exchange of the whole-round protocol: the HIST kernel has merged this rank's histograms into its exchange
-// block (parity of seq).  Barrier, then every CTA sums its slice of the reduce block over all ranks into the
-// workspace copy the resolve step reads, and clears the slice of the OTHER parity block (every peer has finished
-// reading it: it has arrived at this barrier); the last CTA resolves and takes the rank-major tie offsets.
-__global__ void __launch_bounds__(1024, 1)
-auction_peer_exchange_kernel(AuctionPtrs p, long long N, int K, long long jpw, PeerCtx peers, int seq) {
-    pdl_launch_dependents();
-    pdl_wait();
-    __shared__ int s_mode, s_pass;
-    const int tid = threadIdx.x, NT = blockDim.x, par = seq & 1;
-    if (tid == 0) { s_mode = p.st->mode; s_pass = p.st->passes; }
-    __syncthreads();
-    if (s_mode != MODE_HIST) return;
-    const int RB = K * AUC_W + 2 * K;                          // histograms + above + gap (the bid counters travel apart)
-    if (!peer_barrier(peers, 1, seq, blockIdx.x == 0)) {
-        if (tid == 0) { p.st->error = 1; p.st->mode = MODE_DONE; p.st->done = 1; }
-        return;
-    }
-    const unsigned int* mine = peer_hist(peers, peers.rank, K, par);
-    unsigned int* other = peer_hist(peers, peers.rank, K, par ^ 1);
-    for (int i = blockIdx.x * NT + tid; i < RB; i += gridDim.x * NT) {
-        unsigned int acc = __ldcg(mine + i);
-#pragma unroll
-        for (int r = 0; r < PEER_MAX; ++r)                     // all peers' loads in flight together
-            if (r < peers.world && r != peers.rank) acc += __ldcv(peer_hist(peers, r, K, par) + i);
-        p.hist_g[i] = acc;
-        other[i] = 0u;
-    }
-    if (!auction_last_cta(p.ticket)) return;
-    const int this_pass = s_pass;
-    auction_resolve_body(p, N, K, jpw, MODE_HIST);
-    __syncthreads();
-    for (int w = tid; w < K; w += NT) {                        // workers THIS pass resolved (see auction_resolve_peer_kernel)
-        if (p.res_pass[w] != this_pass || p.tkey[w] < 0) continue;
-        const int base = p.win_base[w], hbase = p.win_hbase[w], nlo = p.win_nlo[w], tk = p.tkey[w];
-        const int bin = tk >= hbase ? nlo + tk - hbase : tk - base;
-        unsigned int part[PEER_MAX];
-#pragma unroll
-        for (int r = 0; r < PEER_MAX; ++r)
-            part[r] = (r < peers.rank) ? __ldcv(peer_hist(peers, r, K, par) + (size_t)w * AUC_W + bin) : 0u;
-        unsigned int off = 0;
-#pragma unroll
-        for (int r = 0; r < PEER_MAX; ++r) off += part[r];
-        p.rank_off[w] = off;
-    }
-}
-
-// After a resolve that leaves every worker resolved: per-CTA exclusive prefix of the number of
-// values equal to the threshold (bin tkey-base of the per-CTA dumps), and the window predicted for
-// the values after this round's cost update.  Grid = K CTAs.
+// Step-by-step flow (rqk_auction_resolve), after a resolve that leaves every worker resolved: per-CTA exclusive
+// prefix of the number of values equal to the threshold (bin tkey-base of the per-CTA dumps).  Grid = K CTAs.
 __global__ void __launch_bounds__(AUC_MAX_CTAS, 1)
 auction_tieprefix_kernel(AuctionPtrs p, int K, int G) {
     pdl_launch_dependents();
@@ -2541,8 +2393,8 @@ static int auction_prepare(int64_t n, int64_t ld, int32_t k, void* workspace, si
 }
 
 // Enqueues the kernels of one pass; the device-side state machine makes those whose turn it is not return at
-// once.  which: bit 0 window sampling, bit 1 HIST, bit 2 BID (list replay + S scan), bit 3 tie prefix (between
-// HIST and BID; only meaningful with fused resolve).  fused: the last CTA of a pass kernel runs the resolve step.
+// once.  which: bit 0 window sampling, bit 1 HIST, bit 2 BID (list replay + S scan), bit 3 merge + resolve (between
+// HIST and BID; fused only).  fused: HIST dumps per CTA and the last CTA of a bidding kernel runs the resolve step.
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_round_kernel(void (*kernel)(KArgs...), unsigned grid, unsigned block, size_t smem,
                                        cudaStream_t stream, bool pdl, Args... args) {
@@ -2590,7 +2442,7 @@ static int auction_launch(const AuctionArgs& a, const void* scores_t, int64_t ld
     if (which & 1)
         RQK_CUDA_OK(launch_round_kernel(auction_sample_kernel, (unsigned)k, (unsigned)AUC_SAMPLE_THREADS, 0, stream, pdl, (const __half*)scores_t,
                                         (long long)ld, (long long)n, (int)k, (long long)(n_global / k), a.p,
-                                        (unsigned short*)nullptr, 0, (const unsigned short*)nullptr, 0, 1, PeerCtx{}, 0, -1));
+                                        (unsigned short*)nullptr, 0, (const unsigned short*)nullptr, 0, 1, PeerCtx{}, 0));
     if (which & 2) {
         static bool hs_set[RQK_MAX_DEVICES] = {};
         const size_t hs = HistSmem::TOTAL;
@@ -2602,13 +2454,9 @@ static int auction_launch(const AuctionArgs& a, const void* scores_t, int64_t ld
                                         (const __half*)scores_t, (long long)ld, (long long)n, (int)k, a.J, spc, a.p,
                                         (long long)n_global, fused));
     }
-    if (which & 8) {
-        if (fused)      // HIST only dumped: merge + resolve + tie prefix, one CTA per worker
-            RQK_CUDA_OK(launch_round_kernel(auction_merge_resolve_kernel, (unsigned)k, (unsigned)AUC_MAX_CTAS, 0, stream, pdl,
-                                            a.p, (int)k, a.G, (long long)(n_global / k), spc, auction_list_refine_ok() ? 1 : 0));
-        else
-            RQK_CUDA_OK(launch_round_kernel(auction_tieprefix_kernel, (unsigned)k, (unsigned)AUC_MAX_CTAS, 0, stream, pdl, a.p, (int)k, a.G));
-    }
+    if (which & 8)      // HIST only dumped: merge + resolve + tie prefix, one CTA per worker
+        RQK_CUDA_OK(launch_round_kernel(auction_merge_resolve_kernel, (unsigned)k, (unsigned)AUC_MAX_CTAS, 0, stream, pdl,
+                                        a.p, (int)k, a.G, (long long)(n_global / k), spc, auction_list_refine_ok() ? 1 : 0));
     if (which & 4) {
         RQK_CUDA_OK(launch_round_kernel(auction_bidlist_kernel, (unsigned)a.G, (unsigned)AUC_THREADS, 0, stream, pdl,
                                         (const __half*)scores_t, (long long)ld, (long long)n, (int)k, a.J, spc, a.p,
@@ -2680,7 +2528,7 @@ int rqk_auction_init(int64_t n, int64_t ld, int32_t k, const void* minmax_keys, 
 // The device-side state machine decides what the pass is: three kernels are enqueued and two of them
 // return at once - window sampling (only when windows are cold and the jobs are not sharded), the
 // streaming HIST kernel, the tiled BID kernel.  `which` (0 = all) restricts the launch to a subset
-// (bit 0 sample, bit 1 HIST, bit 2 BID) so that a caller can time one kernel alone.
+// (bit 0 sample, bit 1 HIST, bit 2 BID, bit 3 merge + resolve with bit 4) so that a caller can time one kernel alone.
 int rqk_auction_pass(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, int32_t which,
                      void* workspace, size_t workspace_bytes, void* stream_) {
     using namespace rqk;
@@ -2694,10 +2542,11 @@ int rqk_auction_pass(const void* scores_t, int64_t ld, int64_t n, int32_t k, int
     // bit 4: the kernels of the single-GPU driver's flow (HIST dumps per CTA, bit 3 = merge + resolve + tie prefix, the
     // bidding kernel's last CTA resolves) - timing and tests of exactly what rqk_auction chains; unsharded jobs only
     const int fused = (which & 16) && n_global == n ? 1 : 0;
+    if ((which & 8) && !fused) return fail(RQK_ERR_ARG, "rqk_auction_pass: bit 3 (merge + resolve) needs bit 4 and unsharded jobs%s");
     return auction_launch(a, scores_t, ld, n, k, n_global, which & 15, fused, (cudaStream_t)stream_);
 }
 
-// Sharded window sampling, step 1: keys of `count` (<= 4096) evenly strided local jobs per worker -> out [k][count]
+// Sharded window sampling, step 1: keys of `count` (<= 8192) evenly strided local jobs per worker -> out [k][count]
 // (uint16 fp16 keys).  Writes nothing unless the state machine wants a sample (then `out` is untouched and the
 // window step ignores it), so the host may call both steps unconditionally before every pass.
 int rqk_auction_sample_collect(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, void* out,
@@ -2708,13 +2557,13 @@ int rqk_auction_sample_collect(const void* scores_t, int64_t ld, int64_t n, int3
     if (rc) return rc;
     if (!scores_t || !out || count < 1 || count > AUC_SAMPLE) return fail(RQK_ERR_ARG, "rqk_auction_sample_collect: bad argument%s");
     auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, (cudaStream_t)stream_>>>((const __half*)scores_t, ld, n, k, n_global / k, a.p,
-                                                                  (unsigned short*)out, count, nullptr, 0, 1, PeerCtx{}, 0, -1);
+                                                                  (unsigned short*)out, count, nullptr, 0, 1, PeerCtx{}, 0);
     RQK_LAUNCH_OK();
     return 0;
 }
 
 // Sharded window sampling, step 2: keys [parts][k][count] = the all-gathered samples of every rank, exactly as an
-// all-gather of step 1's outputs lays them out (parts * count <= 4096).
+// all-gather of step 1's outputs lays them out (parts * count <= 8192).
 int rqk_auction_sample_window(int64_t n, int64_t ld, int32_t k, int64_t n_global, const void* keys, int32_t count,
                               int32_t parts, void* workspace, size_t workspace_bytes, void* stream_) {
     using namespace rqk;
@@ -2724,7 +2573,7 @@ int rqk_auction_sample_window(int64_t n, int64_t ld, int32_t k, int64_t n_global
     if (!keys || count < 1 || parts < 1 || (int64_t)count * parts > AUC_SAMPLE)
         return fail(RQK_ERR_ARG, "rqk_auction_sample_window: bad argument%s");
     auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, (cudaStream_t)stream_>>>(nullptr, ld, n_global, k, n_global / k, a.p, nullptr, 0,
-                                                                  (const unsigned short*)keys, count * parts, count, PeerCtx{}, 0, -1);
+                                                                  (const unsigned short*)keys, count * parts, count, PeerCtx{}, 0);
     RQK_LAUNCH_OK();
     return 0;
 }
@@ -2748,8 +2597,8 @@ int rqk_auction_resolve(int64_t n, int64_t ld, int32_t k, int64_t n_global, int3
 
 // ---- peer-memory sharding (DESIGN.md section 4): the exchange is inside the kernels ----
 // peers: HOST array of `world` device pointers, peers[r] = rank r's exchange block (rqk_auction_peer_bytes(k_max)
-// bytes of symmetric memory, zeroed once before first use) as mapped into THIS process; seq: a number that every
-// rank increases by one per call of either function (flags are never reset).
+// bytes of symmetric memory, zeroed once before first use) as mapped into THIS process.  Its flags are never reset:
+// sequence numbers only grow, over all auctions that share the block.
 size_t rqk_auction_peer_bytes(int32_t k) { return rqk::peer_bytes(k); }
 
 static int peer_ctx(const void* const* peers, int32_t world, int32_t rank, rqk::PeerCtx* c, const char* who) {
@@ -2764,37 +2613,11 @@ static int peer_ctx(const void* const* peers, int32_t world, int32_t rank, rqk::
     return 0;
 }
 
-// Window sampling of a sharded job: local samples into the own exchange block, flag barrier, windows from the union.
-int rqk_auction_peer_sample(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, int32_t count,
-                            const void* const* peers, int32_t world, int32_t rank, int32_t seq, void* workspace,
-                            size_t workspace_bytes, void* stream_) {
-    using namespace rqk;
-    AuctionArgs a;
-    int rc = auction_prepare(n, ld, k, workspace, workspace_bytes, &a, "rqk_auction_peer_sample");
-    if (rc) return rc;
-    PeerCtx c;
-    if ((rc = peer_ctx(peers, world, rank, &c, "rqk_auction_peer_sample"))) return rc;
-    if (!scores_t || count < 1 || (int64_t)count * world > AUC_SAMPLE) return fail(RQK_ERR_ARG, "rqk_auction_peer_sample: bad argument%s");
-    cudaStream_t stream = (cudaStream_t)stream_;
-    unsigned short* mine = reinterpret_cast<unsigned short*>(c.buf[rank] + peer_sample_off(k)) + (size_t)(seq & 1) * k * AUC_SAMPLE_MAX;
-    auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, stream>>>((const __half*)scores_t, ld, n, k, n_global / k, a.p, mine, count, nullptr, 0, 1,
-                                                  PeerCtx{}, 0, -1);
-    auction_peer_barrier_kernel<<<1, 32, 0, stream>>>(a.p, c, 0, seq);
-    auction_sample_kernel<<<k, AUC_SAMPLE_THREADS, 0, stream>>>(nullptr, ld, n_global, k, n_global / k, a.p, nullptr, 0, nullptr, count * world, count,
-                                                  c, seq & 1, -1);
-    RQK_LAUNCH_OK();
-    return 0;
-}
-
-int rqk_auction_peer_resolve(int64_t n, int64_t ld, int32_t k, int64_t n_global, int32_t expect, const void* const* peers,
-                             int32_t world, int32_t rank, int32_t seq, void* workspace, size_t workspace_bytes, void* stream_);
-
 // One whole ROUND of a sharded job in one call: seven launches chained with programmatic dependent launch (see
 // "whole-round protocol" above).  Sequence numbers: seq0 = the bid-counter exchange of the PREVIOUS round (its
 // resolve runs at the head of this call), seq0+1 the window samples, seq0+2 the threshold histograms; this round's
 // bid counters are exchanged under seq0+3 by the next call (the caller advances its counter by 3 per call and
-// keeps calling until the state reports done).  The hist area of the own exchange block must be zero when an
-// auction starts (rqk_auction_peer_hist_bytes).
+// keeps calling until the state reports done).
 int rqk_auction_peer_round(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, int32_t count,
                            const void* const* peers, int32_t world, int32_t rank, int32_t seq0, void* workspace,
                            size_t workspace_bytes, void* stream_) {
@@ -2813,52 +2636,14 @@ int rqk_auction_peer_round(const void* scores_t, int64_t ld, int64_t n, int32_t 
                                     (int)(seq0 + 1)));
     RQK_CUDA_OK(launch_round_kernel(auction_sample_kernel, (unsigned)k, (unsigned)AUC_SAMPLE_THREADS, 0, stream, pdl, (const __half*)nullptr, (long long)ld,
                                     (long long)n_global, (int)k, (long long)(n_global / k), a.p, (unsigned short*)nullptr, 0,
-                                    (const unsigned short*)nullptr, (int)(count * world), (int)count, c, (int)((seq0 + 1) & 1),
-                                    (int)(seq0 + 1)));
+                                    (const unsigned short*)nullptr, (int)(count * world), (int)count, c, (int)(seq0 + 1)));
     // HIST dumps per CTA (as in the single-GPU driver); the per-worker publish / resolve kernels exchange the rows
-    static const bool old_xch = [] { const char* e = getenv("RQK_PEER_XCH16"); return e && e[0] == '1'; }();
-    if (!old_xch) {
-        if ((rc = auction_launch(a, scores_t, ld, n, k, n_global, 2, 1, stream, true))) return rc;
-        RQK_CUDA_OK(launch_round_kernel(auction_peer_publish_kernel, (unsigned)k, (unsigned)AUC_MAX_CTAS, 0, stream, pdl, a.p, (int)k,
-                                        a.G, c, (int)(seq0 + 2)));
-        RQK_CUDA_OK(launch_round_kernel(auction_peer_resolve_workers_kernel, (unsigned)k, (unsigned)AUC_MAX_CTAS, 0, stream, pdl, a.p,
-                                        (int)k, a.G, (long long)(n_global / k), c, (int)(seq0 + 2)));
-        if ((rc = auction_launch(a, scores_t, ld, n, k, n_global, 4, 0, stream, true))) return rc;
-        RQK_LAUNCH_OK();
-        return 0;
-    }
-    // RQK_PEER_XCH16=1 (timing comparisons): the HIST kernel merges this rank's histograms with atomics straight into
-    // its exchange block (parity of seq0 + 2), a 16-CTA kernel sums slices over the ranks and its last CTA resolves
-    AuctionArgs ah = a;
-    ah.p.hist_g = reinterpret_cast<unsigned int*>(c.buf[rank] + PEER_FLAGS_BYTES + PEER_TAIL_BYTES) +
-                  (size_t)((seq0 + 2) & 1) * peer_rb_words(k);
-    ah.p.above_g = ah.p.hist_g + (size_t)k * AUC_W;
-    ah.p.gap_g = ah.p.above_g + k;
-    if ((rc = auction_launch(ah, scores_t, ld, n, k, n_global, 2, 0, stream, true))) return rc;
-    RQK_CUDA_OK(launch_round_kernel(auction_peer_exchange_kernel, (unsigned)PEER_XCH_CTAS, 1024u, 0, stream, pdl, a.p,
-                                    (long long)n_global, (int)k, (long long)(n_global / k), c, (int)(seq0 + 2)));
-    if ((rc = auction_launch(a, scores_t, ld, n, k, n_global, 8 | 4, 0, stream, true))) return rc;
-    RQK_LAUNCH_OK();
-    return 0;
-}
-
-// Bytes of the histogram area of an exchange block (it starts at byte 512, after the flag and counter words) that
-// must be zero when an auction starts; the kernels keep it zero from then on.
-size_t rqk_auction_peer_hist_bytes(int32_t k) { return 2 * rqk::peer_rb_words(k) * 4; }
-
-// Resolve step of a sharded job with the rank exchange inside (expect: 0 after a HIST pass, 1 after a BID pass).
-int rqk_auction_peer_resolve(int64_t n, int64_t ld, int32_t k, int64_t n_global, int32_t expect, const void* const* peers,
-                             int32_t world, int32_t rank, int32_t seq, void* workspace, size_t workspace_bytes, void* stream_) {
-    using namespace rqk;
-    AuctionArgs a;
-    int rc = auction_prepare(n, ld, k, workspace, workspace_bytes, &a, "rqk_auction_peer_resolve");
-    if (rc) return rc;
-    PeerCtx c;
-    if ((rc = peer_ctx(peers, world, rank, &c, "rqk_auction_peer_resolve"))) return rc;
-    if (expect != 0 && expect != 1) return fail(RQK_ERR_ARG, "rqk_auction_peer_resolve: expect must be 0 or 1%s");
-    cudaStream_t stream = (cudaStream_t)stream_;
-    auction_resolve_peer_kernel<<<1, 1024, 0, stream>>>(a.p, n_global, k, n_global / k, expect, c, seq);
-    if (expect == 0) auction_tieprefix_kernel<<<k, AUC_MAX_CTAS, 0, stream>>>(a.p, k, a.G);
+    if ((rc = auction_launch(a, scores_t, ld, n, k, n_global, 2, 1, stream, true))) return rc;
+    RQK_CUDA_OK(launch_round_kernel(auction_peer_publish_kernel, (unsigned)k, (unsigned)AUC_MAX_CTAS, 0, stream, pdl, a.p, (int)k,
+                                    a.G, c, (int)(seq0 + 2)));
+    RQK_CUDA_OK(launch_round_kernel(auction_peer_resolve_workers_kernel, (unsigned)k, (unsigned)AUC_MAX_CTAS, 0, stream, pdl, a.p,
+                                    (int)k, a.G, (long long)(n_global / k), c, (int)(seq0 + 2)));
+    if ((rc = auction_launch(a, scores_t, ld, n, k, n_global, 4, 0, stream, true))) return rc;
     RQK_LAUNCH_OK();
     return 0;
 }

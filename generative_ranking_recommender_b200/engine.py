@@ -138,7 +138,6 @@ class ShardGroup:
 
 
 _NO_SHARD = None
-_PEER_STEPS = __import__("os").environ.get("RQK_PEER_MODE", "round") == "steps"
 _SHARD_BATCH = max(1, int(__import__("os").environ.get("RQK_SHARD_BATCH", "3")))   # rounds enqueued per look at the state
 
 
@@ -379,22 +378,10 @@ def auction(scores_t: torch.Tensor, n: int, minmax: torch.Tensor,
         # Exchange through peer memory: the sums over ranks happen inside the sampling / resolve kernels
         # (flag barrier + direct reads of the peers' exchange blocks over NVLink); no collective call per round.
         ptrs = peer[2]
-        if not _PEER_STEPS:
-            # the whole-round protocol lets the HIST kernel merge straight into the exchange block: its histogram
-            # area starts every auction zeroed (every rank is past the previous auction: an all-reduce lies between)
-            peer[0][512:512 + int(L.rqk_auction_peer_hist_bytes(k))].zero_()
         count = max(SAMPLE_JOBS // shard.world, 1)
         for _ in range(0, 5000, batch):
             for _q in range(batch):
-                if _PEER_STEPS:          # the exchange + resolve as their own 1-CTA kernels (debugging / timing)
-                    s0 = shard.take_seq(3)
-                    sess.peer_sample(count, ptrs, shard.world, shard.rank, s0 + 1)
-                    sess.do_pass(2)
-                    sess.peer_resolve(0, ptrs, shard.world, shard.rank, s0 + 2)
-                    sess.do_pass(4)
-                    sess.peer_resolve(1, ptrs, shard.world, shard.rank, s0 + 3)
-                else:
-                    sess.peer_round(count, ptrs, shard.world, shard.rank, shard.take_seq(3))
+                sess.peer_round(count, ptrs, shard.world, shard.rank, shard.take_seq(3))
             if finished(_ // batch):
                 info = sess.poll()
                 break
@@ -466,7 +453,7 @@ class AuctionSession:
 
     def sample_window(self, keys: torch.Tensor):
         """Step 2: keys int16 [world, k, count] = the all-gather of every rank's step-1 output (world * count <=
-        4096); [k, count] is accepted for a single part."""
+        8192); [k, count] is accepted for a single part."""
         if keys.dim() == 2:
             keys = keys.unsqueeze(0)
         self._keys = keys.contiguous()
@@ -474,17 +461,9 @@ class AuctionSession:
         _call(self.dev, self.L.rqk_auction_sample_window, self.n, self.ld, self.k, self.n_global, _ptr(self._keys), int(count),
                                                int(parts), *self._args(), _stream(self.dev))
 
-    def peer_sample(self, count: int, ptrs, world: int, rank: int, seq: int):
-        _call(self.dev, self.L.rqk_auction_peer_sample, _ptr(self.s), self.ld, self.n, self.k, self.n_global, int(count),
-                                             ptrs, world, rank, seq, *self._args(), _stream(self.dev))
-
     def peer_round(self, count: int, ptrs, world: int, rank: int, seq0: int):
         _call(self.dev, self.L.rqk_auction_peer_round, _ptr(self.s), self.ld, self.n, self.k, self.n_global, int(count), ptrs,
                                             world, rank, seq0, *self._args(), _stream(self.dev))
-
-    def peer_resolve(self, expect: int, ptrs, world: int, rank: int, seq: int):
-        _call(self.dev, self.L.rqk_auction_peer_resolve, self.n, self.ld, self.k, self.n_global, expect, ptrs, world, rank, seq,
-                                              *self._args(), _stream(self.dev))
 
     def resolve(self, expect: int = -1):
         """expect: -1, or 0 / 1 = act only if a HIST / BID pass has just run."""

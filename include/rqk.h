@@ -92,13 +92,13 @@ int rqk_auction_init(int64_t n, int64_t ld, int32_t k, const void* minmax_keys, 
                      size_t workspace_bytes, void* stream);
 int rqk_auction_pass(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, int32_t which,
                      void* workspace, size_t workspace_bytes, void* stream);
-/* which: 0 = sample + HIST + BID; else bit0 window sampling, bit1 HIST, bit2 BID, bit3 tie prefix.  Followed by
- * rqk_auction_resolve this is the step-by-step flow (the HIST pass merges its histograms into the reduce block).
+/* which: 0 = sample + HIST + BID; else bit0 window sampling, bit1 HIST, bit2 BID.  Followed by rqk_auction_resolve
+ * this is the step-by-step flow (the HIST pass merges its histograms into the reduce block).
  * bit4 (unsharded jobs): the kernels exactly as rqk_auction chains them - the HIST pass dumps its histograms per CTA,
- * bit3 is then the merge kernel (one CTA per worker: sum of the dumps, threshold, tie prefix, state transition) and
- * the bidding kernel's last CTA resolves the round; no rqk_auction_resolve calls in that flow. */
+ * bit3 is the merge kernel (one CTA per worker: sum of the dumps, threshold, tie prefix, state transition) and the
+ * bidding kernel's last CTA resolves the round; no rqk_auction_resolve calls in that flow.  bit3 requires bit4. */
 /* sharded jobs: every rank samples `count` of its jobs per worker (uint16 fp16 keys, [k][count]); the host
- * all-gathers them into [k][world*count] (<= 4096) and every rank places identical windows from the union */
+ * all-gathers them into [k][world*count] (<= 8192) and every rank places identical windows from the union */
 int rqk_auction_sample_collect(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, void* out,
                                int32_t count, void* workspace, size_t workspace_bytes, void* stream);
 int rqk_auction_sample_window(int64_t n, int64_t ld, int32_t k, int64_t n_global, const void* keys, int32_t count,
@@ -109,19 +109,11 @@ int rqk_auction_tie_offset(int64_t n, int64_t ld, int32_t k, const int32_t* tota
                            void* workspace, size_t workspace_bytes, void* stream);
 /* Jobs sharded over GPUs, exchange through peer memory instead of NCCL (DESIGN.md section 4).  peers: HOST array
  * of `world` (<= 8) device pointers, peers[r] = rank r's exchange block of rqk_auction_peer_bytes(k_max) bytes of
- * symmetric memory (zeroed once) as mapped into this process; seq: increased by one per call by every rank. */
+ * symmetric memory (zeroed once) as mapped into this process; seq0: increased by 3 per call by every rank. */
 size_t rqk_auction_peer_bytes(int32_t k);
-/* bytes [512, 512 + this) of an exchange block must be zero when an auction that uses rqk_auction_peer_round starts */
-size_t rqk_auction_peer_hist_bytes(int32_t k);
-int rqk_auction_peer_sample(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, int32_t count,
-                            const void* const* peers, int32_t world, int32_t rank, int32_t seq, void* workspace,
-                            size_t workspace_bytes, void* stream);
 int rqk_auction_peer_round(const void* scores_t, int64_t ld, int64_t n, int32_t k, int64_t n_global, int32_t count,
                            const void* const* peers, int32_t world, int32_t rank, int32_t seq0, void* workspace,
                            size_t workspace_bytes, void* stream);   /* a whole round (7 launches): seq0 = the previous round's bid counters, seq0+1 samples, seq0+2 histograms */
-int rqk_auction_peer_resolve(int64_t n, int64_t ld, int32_t k, int64_t n_global, int32_t expect,
-                             const void* const* peers, int32_t world, int32_t rank, int32_t seq, void* workspace,
-                             size_t workspace_bytes, void* stream);
 int rqk_auction_poll(int64_t n, int64_t ld, int32_t k, void* workspace, size_t workspace_bytes,
                      rqk_auction_info* info /*HOST*/, void* stream);   /* synchronises */
 int rqk_auction_finalize(int64_t n, int64_t ld, int32_t k, void* workspace, size_t workspace_bytes, int32_t* assign,

@@ -289,12 +289,12 @@ def test_sharded_auction_protocol_single_gpu_emulation(dev, engine, n, k, split,
     assert infos[0].rounds == ref.rounds
 
 
-@pytest.mark.parametrize("whole_round", [False, True])
 @pytest.mark.parametrize("n,k", [(4100, 16), (20010, 128), (12900, 256)])
-def test_peer_exchange_protocol_single_rank(dev, engine, n, k, bid_path, whole_round):
-    """The peer-memory form of the sharded protocol (exchange inside the sampling / resolve kernels) with a world of
-    one rank: its own exchange block is the only peer.  (Two ranks cannot be emulated on one GPU: their kernels
-    would wait for each other on one stream; tools/dist_check.py runs the real thing on 2 GPUs.)"""
+def test_peer_exchange_protocol_single_rank(dev, engine, n, k, bid_path):
+    """The peer-memory form of the sharded protocol (one call per round: seven chained launches, exchanges inside
+    the kernels) with a world of one rank: its own exchange block is the only peer.  (Two ranks cannot be emulated
+    on one GPU: their kernels would wait for each other on one stream; tools/dist_check.py runs the real thing on
+    2 GPUs.)"""
     import ctypes
     rng = np.random.default_rng(n)
     x = O.synth_mix(n, 64, seed=n, modes=max(8, k))
@@ -308,14 +308,7 @@ def test_peer_exchange_protocol_single_rank(dev, engine, n, k, bid_path, whole_r
     sess.init(_mm(st, n))
     seq, info = 0, None
     for _ in range(1500):
-        if whole_round:                 # one call per round: seven chained launches, exchanges inside the kernels
-            sess.peer_round(4096, ptrs, 1, 0, seq)
-        else:                           # step functions: exchange + resolve as their own 1-CTA kernels
-            sess.peer_sample(4096, ptrs, 1, 0, seq + 1)
-            sess.do_pass(2)
-            sess.peer_resolve(0, ptrs, 1, 0, seq + 2)
-            sess.do_pass(4)
-            sess.peer_resolve(1, ptrs, 1, 0, seq + 3)
+        sess.peer_round(4096, ptrs, 1, 0, seq)
         seq += 3
         info = sess.poll()
         if info.done:
