@@ -6,8 +6,9 @@
 //           (:428, :654, :660).  These are the ids train() returns and the jsonl holds.
 //   mode 1  "predict()":   as the reference's predict(): middle levels add fl32(+10000) to every
 //           centre outside the block of the previous id (:1210-1219; with directly trained centres
-//           that is every centre unless the previous id is 0 - SURVEY.md F8), id % need (:1231), and
-//           the residual comes from the UNWEIGHTED running data (:577).
+//           that is every centre unless the previous id is 0 - SURVEY.md F8), and the residual comes
+//           from the UNWEIGHTED running data (:577).  The reference's id % need (:1231) is the identity
+//           when ks[l] == needs[l], which mode 1 requires at the masked levels (else RQK_ERR_UNSUPPORTED).
 //
 // This is the general path: a row-chunked chain of the tcgen05 score pass (argmin only, no score matrix) and the
 // residual kernel per level; the running residual lives in a chunk-sized scratch so X itself is read once per level.
@@ -52,6 +53,12 @@ int rqk_encode(const float* x, int64_t n, int32_t dim, int32_t levels, const voi
     if (!x || !centers || !ks || !needs || !group_end || !ids || !workspace) return fail(RQK_ERR_ARG, "rqk_encode: null pointer%s");
     if (levels < 1 || levels > 16) return fail(RQK_ERR_UNSUPPORTED, "rqk_encode: levels=%s%lld outside [1,16]", "", levels);
     if (mode != 0 && mode != 1) return fail(RQK_ERR_ARG, "rqk_encode: mode=%s%lld must be 0 or 1", "", mode);
+    // predict()'s id % need (:1231) is not applied by the score epilogues, so a masked level must have ks == needs
+    // (a recursive middle layer goes through the host's block-by-block chain instead)
+    if (mode == 1)
+        for (int l = 1; l < levels - 1; ++l)
+            if (needs[l] != ks[l])
+                return fail(RQK_ERR_UNSUPPORTED, "rqk_encode: mode 1 needs ks[l] == needs[l] at masked level l=%s%lld", "", l);
     int kmax = 1;
     for (int l = 0; l < levels; ++l) kmax = ks[l] > kmax ? ks[l] : kmax;
     if (workspace_bytes < rqk_encode_workspace_bytes(n, dim, kmax))

@@ -151,8 +151,10 @@ int rqk_masked_argmin(const float* dist, int64_t n, int32_t k, const int32_t* gr
 int rqk_gather_rows(const float* x, int32_t dim, const int64_t* rows, int32_t nrows, float* out, void* stream);
 
 /* ---- multi-level encode ----------------------------------------------------------------------
- * hierarchical_rq_kmeans.py:539-581 predict (mode 1, incl. the +10000 masking of :1210-1219 and
- * id % need :1231) and the id chain train() emits (mode 0: :654 + :660 per level).
+ * hierarchical_rq_kmeans.py:539-581 predict (mode 1, incl. the +10000 masking of :1210-1219) and the
+ * id chain train() emits (mode 0: :654 + :660 per level).  Mode 1 requires ks[l] == needs[l] at the
+ * masked levels 0 < l < levels-1, where the reference's id % need (:1231) is the identity; other shapes
+ * (a recursive middle layer) return RQK_ERR_UNSUPPORTED.
  * centers / weights: HOST arrays [levels] of device pointers (weights[l] NULL = all ones);
  * ks / needs: HOST int32 [levels]; ids: int32 [levels][n].
  */
