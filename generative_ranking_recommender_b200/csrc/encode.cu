@@ -12,7 +12,7 @@
 //
 // This is the general path: a row-chunked chain of the tcgen05 score pass (argmin only, no score matrix) and the
 // residual kernel per level; the running residual lives in a chunk-sized scratch so X itself is read once per level.
-// It takes per-group weights, several dim-groups and any cluster count <= 256.  Unit weights + one dim-group (what
+// It takes per-group weights, several dim-groups and any cluster count <= 4096 (the score pass's limit).  Unit weights + one dim-group (what
 // train_semantic_ids.py runs) go through the single tensor-core kernel of encode_fused.cu instead (rqk_encode_fused),
 // which reads X once and never materialises a residual; the two are compared with each other and with the oracle in
 // tests/test_gpu_parity.py::test_fused_encode_matches_oracle_chain.

@@ -16,7 +16,7 @@ int score_pass_dispatch(const float* x, long long n, int dim, const float* cente
                         int flags, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
     if (!x || !centers || !workspace) return fail(RQK_ERR_ARG, "rqk_score_pass: null pointer%s");
     if (n < 0 || n > 0x7fffffffLL) return fail(RQK_ERR_ARG, "rqk_score_pass: n=%s%lld outside [0,2^31)", "", n);
-    if (k < 1 || k > 256) return fail(RQK_ERR_UNSUPPORTED, "rqk_score_pass: k=%s%lld outside [1,256]", "", k);
+    if (k < 1 || k > 4096) return fail(RQK_ERR_UNSUPPORTED, "rqk_score_pass: k=%s%lld outside [1,4096]", "", k);
     if (dim < 32 || dim % 32 != 0 || dim > 4096) return fail(RQK_ERR_UNSUPPORTED, "rqk_score_pass: dim=%s%lld must be a multiple of 32 in [32,4096]", "", dim);
     if (o_in.scores_t && (o_in.ld < n || o_in.ld % 128 != 0)) return fail(RQK_ERR_ARG, "rqk_score_pass: ld=%s%lld must be a multiple of 128 and >= n", "", o_in.ld);
     if (((uintptr_t)x & 15) || ((uintptr_t)centers & 15)) return fail(RQK_ERR_ARG, "rqk_score_pass: x and centers must be 16-byte aligned%s");

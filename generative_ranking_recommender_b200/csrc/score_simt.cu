@@ -153,6 +153,8 @@ __global__ void minmax_init_kernel(unsigned int* mm) {
 
 int score_pass_simt(const float* x, long long n, int dim, const float* c, int K, float* x2, float* c2,
                     const ScoreOut& o, cudaStream_t stream) {
+    // the whole centroid block of a k-step sits in shared memory and a thread holds 16 columns per row
+    if (K > 256) return fail(RQK_ERR_UNSUPPORTED, "score_pass_simt: the CUDA-core cross-check takes k <= 256, got %s%lld", "", K);
     if (n == 0) return 0;
     row_sqnorm_kernel<<<(unsigned)ceil_div<long long>(n * 32, 256), 256, 0, stream>>>(x, n, dim, x2);
     row_sqnorm_kernel<<<(unsigned)ceil_div<long long>((long long)K * 32, 256), 256, 0, stream>>>(c, K, dim, c2);

@@ -12,9 +12,9 @@ on sm_100a kernels through `balancekmeans.KMeans` and `engine`; the data stays o
 and the per-level residual overwrites the level's input in place (the reference keeps three N x D
 copies per level).  The two strategies of the shipped PROD config's shape (layer_clusters != need_clusters) run on
 the same kernels: the recursive middle layer (:671-752, :839-904) and the last layer's two balanced fits + match
-matrix (:754-837, :906-1086).  What stays out: layers with 512 or more clusters (`half=True`, the fp16-cdist
-regime of `pairwise_distance_half`; the kernels take K <= 256), which raise NotImplementedError rather than running
-somewhere else.
+matrix (:754-837, :906-1086).  What stays out: fits with 512 or more clusters (`half=True`, the fp16-cdist
+regime of `pairwise_distance_half`; the fit's auction takes K <= 256), which raise NotImplementedError rather than
+running somewhere else.  Scoring (predict, the match matrix, the last layer's 2K candidates) takes up to 4096 centres.
 """
 from __future__ import annotations
 

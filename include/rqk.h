@@ -37,7 +37,8 @@ int rqk_device_check(int device);
  * balancekmeans/__init__.py:576-603 pairwise_distance_full (torch.cdist :596), fused with its
  * consumers: (-D).half() + transpose (:29,:40), max/min for eps (:33), argmin (:312,:328,:528),
  * bincount (:329).  tcgen05 3xTF32, TMA-staged; the N x K fp32 matrix is never written unless
- * `dist` is given.  x [n][dim] fp32, centers [k][dim] fp32, 1 <= k <= 256, dim % 32 == 0.
+ * `dist` is given.  x [n][dim] fp32, centers [k][dim] fp32, 1 <= k <= 4096, dim % 32 == 0.
+ * k > 256 is scored in phases of 256 centres (same outputs; bit1 takes k <= 256 only).
  *   scores_t    [k][ld] fp16 = half(-dist), ld multiple of 128 >= n, columns >= n set to -inf   (or NULL)
  *   argmin      int32 [n]                                                                      (or NULL)
  *   best2       fp32 [n][2] smallest and second-smallest distance                              (or NULL)
