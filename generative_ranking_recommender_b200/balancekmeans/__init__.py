@@ -9,8 +9,11 @@ every torch library call on the path replaced by sm_100a kernels from librqk_sm1
   auction_lap_half         :12-140
   pairwise_distance_full   :576-603
 
+`fit` and `fit_by_min_loss` take any n_clusters <= 512 with half=False (the reference's full-precision regime: it
+passes half=True from 512 clusters on in the hierarchy, and above 512 in the Simplified generator).
+
 What is NOT here, on purpose (SURVEY.md section 2): cosine / soft-DTW distances, `pairwise_distance_half`
-and `auction_lap_full` are unreachable from the `[128,128,256]` hot path and raise NotImplementedError
+(half=True) and `auction_lap_full` are unreachable from the `[128,128,256]` hot path and raise NotImplementedError
 instead of silently running somewhere else.  There is no CPU path: a CPU device raises.
 """
 from __future__ import annotations

@@ -34,7 +34,7 @@
 //            retain hack (:86-87) and counter>1000 fallback (:88-89) per job, column max with first-argmax (:104),
 //            cost / owner update (:118-123).
 //   S-scanning fallback  (auction_pass_kernel, after a survivor-list overflow) the same bidding round from tiles of
-//            all K workers x 128 (K<=128) or 64 jobs, bulk-copied into shared memory through a 3-deep ring.
+//            all K workers x 128 (K<=128) or 64 jobs, bulk-copied into shared memory through a 3-deep ring (K <= 512).
 // In the single-GPU driver the last CTA of the bidding kernel runs the resolve step (termination, frozen detection,
 // next state).  With the jobs sharded over GPUs the same kernels run on every rank's shard, and the sums over ranks
 // happen either inside the kernels over peer memory (rqk_auction_peer_round) or through NCCL between step functions.
@@ -69,7 +69,9 @@ constexpr int AUC_SUB = 4096;      // jobs whose cost / owner are staged in shar
 constexpr int AUC_QCAP = 256;      // per-warp survivor queue of the HIST kernel (one row segment; = AUC_SEG_CAP)
 constexpr int AUC_SAMPLE_MAX = 8192; // window-sampling jobs per worker (all ranks together)
 constexpr int AUC_SEG_CAP = 256;   // survivor-list entries per (sub-range, worker); ~60 expected
-constexpr int AUC_KH = 128;        // workers per histogram half of the HIST kernel
+constexpr int AUC_KH = 128;        // workers per histogram slice of the HIST kernel
+constexpr int AUC_KMAX = AUC_THREADS; // workers of an auction at most: the HIST kernel's ordered compaction gives each
+                                      // worker one thread; also keeps owner (int16), act (u16) and ~worker (16 bits) in range
 constexpr int AUC_SAMPLE_THREADS = 512; // threads of a window-sampling CTA (2 CTAs per SM: K = 256 in one wave)
 
 enum { MODE_HIST = 0, MODE_BID = 1, MODE_DONE = 2 };
@@ -681,13 +683,18 @@ __device__ __forceinline__ void bulk_g2s(void* dst, const void* src, unsigned by
 // The BID pass.  Per tile (all K workers x J jobs in shared memory, bulk-copied, double buffered): the sweep
 // filters S - cost against each worker's threshold T_w (one HSUB2 + one HSET2 per two elements); the ~1 %
 // survivors, kept as register bitmasks, become bids; column maximum; cost / owner update.
-template <int J>
+// Instances: <128, 128> (K <= 128), <64, 256> (K <= 256), <64, 512> (K <= 512: the 3-deep ring of 512 x 64 jobs is
+// 192 KB).  A warp's rows are swept in groups of MAXR (the survivor bitmasks hold 16 rows): one group up to K = 256,
+// two at K <= 512, each group's bids placed before the next group is swept.
+template <int J, int KMAX>
 __global__ void __launch_bounds__(AUC_THREADS, (J == 128 ? 2 : 1))
 auction_pass_kernel(const __half* __restrict__ S, long long ld, long long N, int K, long long jpw, AuctionPtrs p,
                     long long n_global, int fused) {
     constexpr int CPL = J / 32;           // columns per lane
     constexpr int NH2 = CPL / 2;          // half2 words per lane
-    constexpr int MAXR = 256 / AUC_NW * (J == 128 ? 1 : 2) / 2;   // rows per warp: 8 (K<=128) / 16 (K<=256)
+    constexpr int MAXR = 256 / AUC_NW * (J == 128 ? 1 : 2) / 2;   // rows per warp and group: 8 (K<=128) / 16
+    constexpr int NGRP = (KMAX + AUC_NW * MAXR - 1) / (AUC_NW * MAXR);   // row groups: 1 (K<=256) / 2 (K<=512)
+    static_assert(MAXR * NGRP <= 32, "one flag bit per row of a warp");
     extern __shared__ __align__(16) unsigned char smem_raw[];
     pdl_launch_dependents();
     pdl_wait();
@@ -744,9 +751,9 @@ auction_pass_kernel(const __half* __restrict__ S, long long ld, long long N, int
     __syncthreads();
 
     // per-row sweep filter in registers (the rows of a warp are w = warp + 16 i)
-    unsigned int f2r[MAXR];
+    unsigned int f2r[MAXR * NGRP];
 #pragma unroll
-    for (int i = 0; i < MAXR; ++i) {
+    for (int i = 0; i < MAXR * NGRP; ++i) {
         const int w = warp + AUC_NW * i;
         f2r[i] = (w < K) ? sm.r_lo2[w] : 0x7c007c00u;
     }
@@ -814,109 +821,114 @@ auction_pass_kernel(const __half* __restrict__ S, long long ld, long long N, int
             }
             __syncthreads();                                                 // S1: row flags visible
             const int wf = warp + AUC_NW * lane;
-            flagmask = __ballot_sync(0xffffffffu, lane < MAXR && wf < K && sm.row_flag[wf] != 0);
+            flagmask = __ballot_sync(0xffffffffu, lane < MAXR * NGRP && wf < K && sm.row_flag[wf] != 0);
         }
 
         // ---------------- the sweep: half2 filter; survivors recorded as register bitmasks ----------------
-        // acc[h] bit i      : column 2h   of row warp+16i survives
-        // acc[h] bit 16 + i : column 2h+1 of row warp+16i survives        (rej[h]: same layout, rejected ties)
-        unsigned int acc[NH2], rej[NH2];
+        // acc[h] bit i      : column 2h   of row warp+16(g*MAXR+i) survives
+        // acc[h] bit 16 + i : column 2h+1 of row warp+16(g*MAXR+i) survives        (rej[h]: same layout, rejected ties)
 #pragma unroll
-        for (int h = 0; h < NH2; ++h) { acc[h] = 0; rej[h] = 0; }
-        const unsigned* tile_u = reinterpret_cast<const unsigned*>(tile) + lane * NH2;
+        for (int g = 0; g < NGRP; ++g) {
+            unsigned int acc[NH2], rej[NH2];
 #pragma unroll
-        for (int i = 0; i < MAXR; ++i) {
-            const int w = warp + AUC_NW * i;
-            if (w >= K) break;
-            const __half2 f2 = u2h2(f2r[i]);
-            const unsigned* row = tile_u + (size_t)w * (J / 2);
-            const bool flagged = (flagmask >> i) & 1u;
-            const unsigned int rowbits = (1u << i) | (1u << (16 + i));
-            __half2 v2[NH2];
-            if (!flagged) {
+            for (int h = 0; h < NH2; ++h) { acc[h] = 0; rej[h] = 0; }
+            const unsigned* tile_u = reinterpret_cast<const unsigned*>(tile) + lane * NH2;
 #pragma unroll
-                for (int h = 0; h < NH2; ++h) {
-                    v2[h] = __hsub2(u2h2(row[h]), c2[h]);                    // ownership ignored: the owner's S is only larger
-                    acc[h] |= __hge2_mask(v2[h], f2) & rowbits;
+            for (int i = 0; i < MAXR; ++i) {
+                const int w = warp + AUC_NW * (g * MAXR + i);
+                if (w >= K) break;
+                const __half2 f2 = u2h2(f2r[g * MAXR + i]);
+                const unsigned* row = tile_u + (size_t)w * (J / 2);
+                const bool flagged = (flagmask >> (g * MAXR + i)) & 1u;
+                const unsigned int rowbits = (1u << i) | (1u << (16 + i));
+                __half2 v2[NH2];
+                if (!flagged) {
+#pragma unroll
+                    for (int h = 0; h < NH2; ++h) {
+                        v2[h] = __hsub2(u2h2(row[h]), c2[h]);                    // ownership ignored: the owner's S is only larger
+                        acc[h] |= __hge2_mask(v2[h], f2) & rowbits;
+                    }
+                } else {
+#pragma unroll
+                    for (int h = 0; h < NH2; ++h) {                              // exact values incl. owner entries
+                        unsigned int cr = h22u(c2[h]);
+                        if (sm.colown[lane * CPL + 2 * h] == w) cr &= 0xffff0000u;
+                        if (sm.colown[lane * CPL + 2 * h + 1] == w) cr &= 0x0000ffffu;
+                        v2[h] = __hsub2(u2h2(row[h]), u2h2(cr));
+                        acc[h] |= __hge2_mask(v2[h], f2) & rowbits;
+                    }
                 }
-            } else {
+                if (do_bid) {                                                    // f2 == T_w in a BID pass
+                    unsigned int anye = 0, em[NH2];
 #pragma unroll
-                for (int h = 0; h < NH2; ++h) {                              // exact values incl. owner entries
-                    unsigned int cr = h22u(c2[h]);
-                    if (sm.colown[lane * CPL + 2 * h] == w) cr &= 0xffff0000u;
-                    if (sm.colown[lane * CPL + 2 * h + 1] == w) cr &= 0x0000ffffu;
-                    v2[h] = __hsub2(u2h2(row[h]), u2h2(cr));
-                    acc[h] |= __hge2_mask(v2[h], f2) & rowbits;
+                    for (int h = 0; h < NH2; ++h) { em[h] = __heq2_mask(v2[h], f2); anye |= em[h]; }
+                    const unsigned int seen0 = sm.tie_seen[w];
+                    const long long quota0 = sm.r_take[w];
+                    if ((long long)seen0 >= quota0) {
+                        // the worker's quota of ties was used up by lower job indices: every tie here is rejected
+                        // (owner entries and padding columns are skipped in stage A anyway)
+#pragma unroll
+                        for (int h = 0; h < NH2; ++h) rej[h] |= em[h] & rowbits;
+                    } else if (__any_sync(0xffffffffu, anye != 0)) {
+                        // canonical tie rule: lowest job index first, globally (tieprefix + tiles so far).
+                        // In unflagged rows owner entries cannot tie (the column thread would have flagged the row).
+                        bool eq[CPL];
+                        unsigned int before = 0, total = 0, mine = 0;
+#pragma unroll
+                        for (int e = 0; e < CPL; ++e) {
+                            const int cidx = lane * CPL + e;
+                            eq[e] = ((em[e >> 1] >> ((e & 1) * 16)) & 1u) != 0 && cidx < ncols &&
+                                    (flagged || sm.colown[cidx] != w);
+                            unsigned int mm = __ballot_sync(0xffffffffu, eq[e]);
+                            before += __popc(mm & lt);
+                            total += __popc(mm);
+                        }
+                        const unsigned int seen = sm.tie_seen[w];
+                        const long long quota = sm.r_take[w];
+#pragma unroll
+                        for (int e = 0; e < CPL; ++e) {
+                            if (eq[e]) {
+                                if (!((long long)(seen + before + mine) < quota)) rej[e >> 1] |= 1u << ((e & 1) * 16 + i);
+                                mine++;
+                            }
+                        }
+                        __syncwarp();
+                        if (lane == 0) sm.tie_seen[w] = seen + total;
+                        __syncwarp();
+                    }
                 }
             }
-            if (do_bid) {                                                    // f2 == T_w in a BID pass
-                unsigned int anye = 0, em[NH2];
+
+            if (do_bid) {
+                // ---------------- stage A: survivors -> bids (of this row group) ----------------
 #pragma unroll
-                for (int h = 0; h < NH2; ++h) { em[h] = __heq2_mask(v2[h], f2); anye |= em[h]; }
-                const unsigned int seen0 = sm.tie_seen[w];
-                const long long quota0 = sm.r_take[w];
-                if ((long long)seen0 >= quota0) {
-                    // the worker's quota of ties was used up by lower job indices: every tie here is rejected
-                    // (owner entries and padding columns are skipped in stage A anyway)
-#pragma unroll
-                    for (int h = 0; h < NH2; ++h) rej[h] |= em[h] & rowbits;
-                } else if (__any_sync(0xffffffffu, anye != 0)) {
-                    // canonical tie rule: lowest job index first, globally (tieprefix + tiles so far).
-                    // In unflagged rows owner entries cannot tie (the column thread would have flagged the row).
-                    bool eq[CPL];
-                    unsigned int before = 0, total = 0, mine = 0;
-#pragma unroll
-                    for (int e = 0; e < CPL; ++e) {
-                        const int cidx = lane * CPL + e;
-                        eq[e] = ((em[e >> 1] >> ((e & 1) * 16)) & 1u) != 0 && cidx < ncols &&
-                                (flagged || sm.colown[cidx] != w);
-                        unsigned int mm = __ballot_sync(0xffffffffu, eq[e]);
-                        before += __popc(mm & lt);
-                        total += __popc(mm);
+                for (int h = 0; h < NH2; ++h) {
+                    unsigned int a = acc[h];
+                    while (a) {
+                        const int bpos = __ffs(a) - 1;
+                        a &= a - 1;
+                        const int i = bpos & 15;
+                        const int w = warp + AUC_NW * (g * MAXR + i), col = lane * CPL + 2 * h + (bpos >> 4);
+                        if (col >= ncols) continue;
+                        const int o = sm.colown[col];
+                        const bool own = (o == w);
+                        const bool flagged_row = (flagmask >> (g * MAXR + i)) & 1u;
+                        if (own && !flagged_row) continue;                       // the column thread did it
+                        const __half sv = tile[(size_t)w * J + col];
+                        const __half v = own ? sv : __hsub(sv, __ushort_as_half(sm.colcost[col]));
+                        const __half T = bits2h(sm.r_T2[w] & 0xffffu);
+                        const bool rejected = (rej[h] >> bpos) & 1u;
+                        if (!(__hgt(v, T) || (__heq(v, T) && !rejected))) continue;
+                        if (fallback && w == 0 && o < 0) continue;               // :89 overrides worker 0's own bid
+                        unsigned int bid = h2bits(__hadd(__hsub(v, T), eps));    // :76, two roundings
+                        if (retain && own) bid = eps_bits;                       // :87
+                        if (!own) sm.colviol[col] = 1;                           // fresh bid on a job the bidder does not own
+                        atomicMax(&sm.colmax[col], (bid << 16) | (0xffffu - (unsigned)w));   // :104
                     }
-                    const unsigned int seen = sm.tie_seen[w];
-                    const long long quota = sm.r_take[w];
-#pragma unroll
-                    for (int e = 0; e < CPL; ++e) {
-                        if (eq[e]) {
-                            if (!((long long)(seen + before + mine) < quota)) rej[e >> 1] |= 1u << ((e & 1) * 16 + i);
-                            mine++;
-                        }
-                    }
-                    __syncwarp();
-                    if (lane == 0) sm.tie_seen[w] = seen + total;
-                    __syncwarp();
                 }
             }
         }
-
         if (do_bid) {
-            // ---------------- stage A: survivors -> bids ----------------
-#pragma unroll
-            for (int h = 0; h < NH2; ++h) {
-                unsigned int a = acc[h];
-                while (a) {
-                    const int bpos = __ffs(a) - 1;
-                    a &= a - 1;
-                    const int i = bpos & 15;
-                    const int w = warp + AUC_NW * i, col = lane * CPL + 2 * h + (bpos >> 4);
-                    if (col >= ncols) continue;
-                    const int o = sm.colown[col];
-                    const bool own = (o == w);
-                    const bool flagged_row = (flagmask >> i) & 1u;
-                    if (own && !flagged_row) continue;                       // the column thread did it
-                    const __half sv = tile[(size_t)w * J + col];
-                    const __half v = own ? sv : __hsub(sv, __ushort_as_half(sm.colcost[col]));
-                    const __half T = bits2h(sm.r_T2[w] & 0xffffu);
-                    const bool rejected = (rej[h] >> bpos) & 1u;
-                    if (!(__hgt(v, T) || (__heq(v, T) && !rejected))) continue;
-                    if (fallback && w == 0 && o < 0) continue;               // :89 overrides worker 0's own bid
-                    unsigned int bid = h2bits(__hadd(__hsub(v, T), eps));    // :76, two roundings
-                    if (retain && own) bid = eps_bits;                       // :87
-                    if (!own) sm.colviol[col] = 1;                           // fresh bid on a job the bidder does not own
-                    atomicMax(&sm.colmax[col], (bid << 16) | (0xffffu - (unsigned)w));   // :104
-                }
-            }
             __syncthreads();                                                 // S3: all bids in colmax
 
             // ---------------- highest bid per job, cost/owner update (:104, :118-123) ----------------
@@ -976,10 +988,10 @@ __device__ __forceinline__ uint4 ldg_stream128(const void* ptr) {
 }
 
 // Shared-memory layout with compile-time offsets: with run-time offsets the compiler re-derives the array bases inside
-// the hot loops (64 registers per thread leave no room to keep them).  The histogram holds one half of the workers
-// (AUC_KH rows, 64 KB, so that two CTAs fit on an SM); the per-worker arrays hold all K <= 256.
+// the hot loops (64 registers per thread leave no room to keep them).  The histogram holds one slice of the workers
+// (AUC_KH rows, 64 KB, so that two CTAs fit on an SM); the per-worker arrays hold all K <= KMAX.
+template <int KMAX>
 struct HistSmem {
-    static constexpr int KMAX = 256;
     static constexpr int HIST = 0;                                    // [AUC_KH][W/2] two 16-bit counters per word
     static constexpr int COST = HIST + AUC_KH * AUC_W * 2;            // [HS_SUB] fp16
     static constexpr int OWN = COST + HS_SUB * 2;                     // [HS_SUB] int16
@@ -996,13 +1008,19 @@ struct HistSmem {
     static constexpr int TOTAL = (RSHIFT + KMAX + 15) / 16 * 16;
 };
 
-// K > AUC_KH: the CTA runs its job range once per half of the workers, [0, 128) then [128, K), with the histogram
-// cleared in between.  That keeps the K = 128 register and shared-memory budget (2 CTAs per SM) for every K; the
-// cost / owner staging is repeated per half (6 bytes per job against 256 bytes of S per job and half).
+// K > AUC_KH: the CTA runs its job range once per slice of AUC_KH workers, [0, 128), [128, 256), .. up to K, with the
+// histogram published and cleared in between.  That keeps the K = 128 register and shared-memory budget (2 CTAs per
+// SM) for every K; the cost / owner staging is repeated per slice (6 bytes per job against 256 bytes of S per job and
+// slice).  A slice without an unresolved worker is skipped.
+// Instances: KMAX = 256 (K <= 256: 96 KB of shared memory per CTA) and KMAX = 512 (K <= 512: 104 KB).  Two CTAs of the
+// larger one need a bigger shared-memory carveout (less L1); run at K = 256 it made the bench step 5 % slower (5.33
+// against 5.09 ms on a B200 at 1000 W), so K <= 256 keeps the smaller layout.
+template <int KMAX>
 __global__ void __launch_bounds__(AUC_THREADS, 2)
 auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int K, int J, int spc, AuctionPtrs p,
                     long long n_global, int fused) {
-    using L = HistSmem;
+    static_assert(KMAX <= AUC_KMAX && KMAX % AUC_KH == 0, "one compaction thread per worker, whole slices");
+    using L = HistSmem<KMAX>;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     pdl_launch_dependents();
     // nothing below depends on earlier kernels until pdl_wait(): the histogram is cleared while they finish
@@ -1030,7 +1048,8 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
     short* const own_s = reinterpret_cast<short*>(smem_raw + L::OWN);
     unsigned int* const seg_cnt_s = reinterpret_cast<unsigned int*>(smem_raw + L::SEGCNT);
     unsigned short* const act = reinterpret_cast<unsigned short*>(smem_raw + L::ACT);
-    __shared__ int s_act_off[3], s_any_cold[2], s_wcnt[AUC_NW];
+    constexpr int NSL = KMAX / AUC_KH;                           // worker slices at most
+    __shared__ int s_act_off[NSL + 1], s_any_cold[NSL], s_wcnt[AUC_NW];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const unsigned int lt = (1u << lane) - 1u;
     unsigned short* const wq = reinterpret_cast<unsigned short*>(smem_raw + L::HQ) + warp * AUC_QCAP;
@@ -1043,8 +1062,8 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
     // Rows (workers) of this pass.  A worker whose threshold an earlier pass of the SAME round resolved keeps what
     // that pass produced (threshold, survivor lists, per-CTA dump) and is skipped: after a window miss only the
     // workers that missed are streamed again, spread over the warps (act[] = the unresolved workers, ascending; those
-    // of half h are act[s_act_off[h] .. s_act_off[h + 1])).
-    if (tid < 2) s_any_cold[tid] = 0;
+    // of slice h are act[s_act_off[h] .. s_act_off[h + 1])).
+    if (tid < NSL) s_any_cold[tid] = 0;
     for (int i = tid; i < K; i += AUC_THREADS) {
         sm.above[i] = 0;
         sm.gap[i] = 0;
@@ -1057,7 +1076,8 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
         sm.r_lo2[i] = lob | (lob << 16);
     }
     __syncthreads();
-    {   // ordered compaction (K <= 256 < AUC_THREADS: one round)
+    {   // ordered compaction: one round, thread i = worker i (K <= AUC_KMAX = AUC_THREADS = 512: the ceiling of this design)
+        static_assert(KMAX / 32 <= AUC_NW, "slices start at warp boundaries");
         const bool a = tid < K && sm.r_shift[tid] != 0xff;
         const unsigned int m = __ballot_sync(0xffffffffu, a);
         if (lane == 0) s_wcnt[warp] = __popc(m);
@@ -1070,24 +1090,23 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
         }
         if (tid == 0) {
             int t = 0;
-            for (int q = 0; q < AUC_NW; ++q) {
-                if (q == AUC_KH / 32) s_act_off[1] = t;
+            for (int q = 0; q < KMAX / 32; ++q) {
+                if (q % (AUC_KH / 32) == 0) s_act_off[q / (AUC_KH / 32)] = t;   // slice q / 4 starts at warp q
                 t += s_wcnt[q];
             }
-            s_act_off[0] = 0;
-            s_act_off[2] = t;
+            s_act_off[NSL] = t;
         }
         __syncthreads();
     }
 
-    int ffh = ff;                                            // the retain fast-forward goes to the first half streamed
+    int ffh = ff;                                            // the retain fast-forward goes to the first slice streamed
     for (int h0 = 0; h0 < K; h0 += AUC_KH) {
         const unsigned short* const acth = act + s_act_off[h0 / AUC_KH];
         const int nact = s_act_off[h0 / AUC_KH + 1] - s_act_off[h0 / AUC_KH];
-        if (nact == 0) continue;                                 // every worker of the half was resolved by an earlier pass
+        if (nact == 0) continue;                                 // every worker of the slice was resolved by an earlier pass
         const int any_cold = s_any_cold[h0 / AUC_KH];            // cold rows take the unpipelined path
         if (h0 > 0) {
-            __syncthreads();                                     // the previous half's histogram has been published
+            __syncthreads();                                     // the previous slice's histogram has been published
             clear_hist();
             __syncthreads();
         }
@@ -1119,7 +1138,7 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
                 own_s[i] = o;
             }
             __syncthreads();
-            // ---- owner entries (value = S): one per job, counted in the owner's half ----
+            // ---- owner entries (value = S): one per job, counted in the owner's slice ----
 #pragma unroll
             for (int it = 0; it < HS_SUB / AUC_THREADS; ++it) {
                 const int i = tid + it * AUC_THREADS;
@@ -1346,7 +1365,7 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
             }
         }
 
-        // ---- publish the half's histogram rows (active rows only) ----
+        // ---- publish the slice's histogram rows (active rows only) ----
         // fused (single-GPU driver): plain stores into the per-CTA dump; auction_merge_resolve_kernel (one CTA per worker,
         // next in the chain) sums them over the CTAs, resolves the worker's threshold and takes the tie prefix - no global
         // atomics here, no serial resolve in a last CTA.  Step-by-step / sharded flows: the per-CTA dump (for the tie
@@ -1365,7 +1384,7 @@ auction_hist_kernel(const __half* __restrict__ S, long long ld, long long N, int
         ffh = 0;
     }
 
-    const int nact_all = s_act_off[2];
+    const int nact_all = s_act_off[NSL];
     for (int a = tid; a < nact_all; a += AUC_THREADS) {
         const int i = act[a];
         if (fused) {
@@ -1397,8 +1416,8 @@ auction_bidlist_kernel(const __half* __restrict__ S, long long ld, long long N, 
     __shared__ __align__(16) unsigned int colmax[AUC_SUB];
     __shared__ __align__(16) short own_s[AUC_SUB];
     __shared__ __align__(16) unsigned char colviol[AUC_SUB];
-    __shared__ unsigned int tie_seen[256];
-    __shared__ int r_take[256], r_tk[256];
+    __shared__ unsigned int tie_seen[AUC_KMAX];
+    __shared__ int r_take[AUC_KMAX], r_tk[AUC_KMAX];
     __shared__ unsigned int s_nwith, s_nviol;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int counter = st.counter;
@@ -2379,8 +2398,8 @@ struct AuctionArgs {
 };
 static int auction_prepare(int64_t n, int64_t ld, int32_t k, void* workspace, size_t workspace_bytes, AuctionArgs* a,
                            const char* who) {
+    if (k < 1 || k > AUC_KMAX) return fail(RQK_ERR_UNSUPPORTED, "%s: k=%lld outside [1,512]", who, k);
     if (!workspace) return fail(RQK_ERR_ARG, "%s: null workspace", who);
-    if (k < 1 || k > 256) return fail(RQK_ERR_UNSUPPORTED, "%s: k=%lld outside [1,256]", who, k);
     if (n < 1) return fail(RQK_ERR_ARG, "%s: n=%lld < 1", who, n);
     if (ld % 128 != 0 || ld < n) return fail(RQK_ERR_ARG, "%s: ld=%lld must be a multiple of 128 and >= n", who, ld);
     size_t need = auction_ws_layout(n, ld, k, &a->p, (char*)workspace);
@@ -2427,13 +2446,13 @@ static int auction_launch(const AuctionArgs& a, const void* scores_t, int64_t ld
     // the single-GPU driver (fused resolve) and the whole-round sharded protocol (`chain`) chain their round kernels
     // with programmatic dependent launch
     const bool pdl = (fused != 0 || chain) && auction_pdl_ok();
-    auto kern = (a.J == 128) ? auction_pass_kernel<128> : auction_pass_kernel<64>;
+    auto kern = (a.J == 128) ? auction_pass_kernel<128, 128> : (k <= 256 ? auction_pass_kernel<64, 256> : auction_pass_kernel<64, 512>);
     // the attribute is per device (and this process may drive several): cache what has been set per device ordinal
     int devi = 0;
     RQK_CUDA_OK(cudaGetDevice(&devi));
     devi &= RQK_MAX_DEVICES - 1;
-    static size_t smem_set[RQK_MAX_DEVICES][2] = {};
-    size_t& cur = smem_set[devi][a.J == 128 ? 0 : 1];
+    static size_t smem_set[RQK_MAX_DEVICES][3] = {};
+    size_t& cur = smem_set[devi][a.J == 128 ? 0 : (k <= 256 ? 1 : 2)];
     if (a.smem > cur) {
         RQK_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)a.smem));
         cur = a.smem;
@@ -2444,13 +2463,15 @@ static int auction_launch(const AuctionArgs& a, const void* scores_t, int64_t ld
                                         (long long)ld, (long long)n, (int)k, (long long)(n_global / k), a.p,
                                         (unsigned short*)nullptr, 0, (const unsigned short*)nullptr, 0, 1, PeerCtx{}, 0));
     if (which & 2) {
-        static bool hs_set[RQK_MAX_DEVICES] = {};
-        const size_t hs = HistSmem::TOTAL;
-        if (!hs_set[devi]) {
-            RQK_CUDA_OK(cudaFuncSetAttribute(auction_hist_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hs));
-            hs_set[devi] = true;
+        static bool hs_set[RQK_MAX_DEVICES][2] = {};
+        const bool wide = k > 256;
+        const auto hk = wide ? auction_hist_kernel<512> : auction_hist_kernel<256>;
+        const size_t hs = wide ? HistSmem<512>::TOTAL : HistSmem<256>::TOTAL;
+        if (!hs_set[devi][wide]) {
+            RQK_CUDA_OK(cudaFuncSetAttribute(hk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)hs));
+            hs_set[devi][wide] = true;
         }
-        RQK_CUDA_OK(launch_round_kernel(auction_hist_kernel, (unsigned)a.G, (unsigned)AUC_THREADS, hs, stream, pdl,
+        RQK_CUDA_OK(launch_round_kernel(hk, (unsigned)a.G, (unsigned)AUC_THREADS, hs, stream, pdl,
                                         (const __half*)scores_t, (long long)ld, (long long)n, (int)k, a.J, spc, a.p,
                                         (long long)n_global, fused));
     }
@@ -2493,7 +2514,8 @@ struct rqk_auction_info {
 
 int rqk_auction_layout_query(int64_t n, int32_t k, rqk_auction_layout* out) {
     using namespace rqk;
-    if (!out || n < 1 || k < 1 || k > 256) return fail(RQK_ERR_ARG, "rqk_auction_layout_query: bad argument%s");
+    if (k < 1 || k > AUC_KMAX) return fail(RQK_ERR_UNSUPPORTED, "rqk_auction_layout_query: k=%s%lld outside [1,512]", "", k);
+    if (!out || n < 1) return fail(RQK_ERR_ARG, "rqk_auction_layout_query: bad argument%s");
     long long ld = round_up<long long>(n, 128);
     size_t ro = 0, to = 0;
     out->total_bytes = (int64_t)auction_ws_layout(n, ld, k, nullptr, nullptr, &ro, &to);

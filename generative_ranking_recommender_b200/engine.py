@@ -23,6 +23,9 @@ from . import _lib, sharding
 from ._lib import AuctionInfo, AuctionLayout, RqkError, check, lib
 
 
+AUCTION_KMAX = 512      # clusters of one balanced fit at most (csrc/auction.cu, AUC_KMAX)
+
+
 def _ptr(t: Optional[torch.Tensor]):
     return ctypes.c_void_p(t.data_ptr()) if t is not None else None
 
@@ -84,7 +87,7 @@ class ShardGroup:
             if self.nccl and self.world <= 8 and os.environ.get("RQK_NO_PEER", "0") != "1":
                 try:
                     import torch.distributed._symmetric_memory as symm
-                    nbytes = int(lib().rqk_auction_peer_bytes(256))
+                    nbytes = int(lib().rqk_auction_peer_bytes(AUCTION_KMAX))   # once per group: fits of any size
                     t = symm.empty(nbytes, dtype=torch.uint8, device=dev)
                     t.zero_()
                     h = symm.rendezvous(t, group=self.group if self.group is not None else self.dist.group.WORLD)

@@ -54,7 +54,8 @@ int rqk_score_pass(const float* x, int64_t n, int32_t dim, const float* centers,
                    float* dist, int32_t flags, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- balanced assignment --------------------------------------------------------------------
- * balancekmeans/__init__.py:12-140 auction_lap_half on the worker-major fp16 score matrix.
+ * balancekmeans/__init__.py:12-140 auction_lap_half on the worker-major fp16 score matrix, 1 <= k <= 512 workers
+ * (every auction entry point returns -4 for any other k before it reads a pointer).
  * Canonical tie rule (the reference leaves it to torch.topk's heap order): among jobs whose value
  * equals a worker's threshold, lowest job index first.  n >= k required (the n < k quirk is the
  * score pass with flags bit0).  rqk_auction() is the single-GPU driver and SYNCHRONISES the stream
